@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — the render hot path on N B200s, one process per GPU.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload c1..c5] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload c1..c5] [--impl ours|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 A "step" is one pass of the hot path over the workload: every scene of the named BASELINE configuration rendered
@@ -51,7 +51,7 @@ UNIT = "Mrays/s"
 def parse_args():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=5)
+    ap.add_argument("--steps", type=positive_int, default=5)
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--workload", default="c5", choices=["c1", "c2", "c3", "c4", "c5"])
@@ -63,7 +63,45 @@ def parse_args():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--cpu-seconds", type=float, default=15.0, help="target CPU time of the cpu_baseline sample")
     ap.add_argument("--ref-seconds", type=float, default=120.0, help="--impl reference: CPU time budget of the whole run")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the images of the last one as DIR/<scene>.npy (see dump_outputs)")
+    args = ap.parse_args()
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs needs --impl ours: the reference arm sizes its spp from a timing probe, so its images differ "
+                 "from run to run")
+    return args
+
+
+def positive_int(s):
+    v = int(s)
+    if v < 1:
+        raise argparse.ArgumentTypeError(f"must be >= 1, got {v}")
+    return v
+
+
+DUMP_BYTES = 60 << 20    # below 64 MB in all, .npy headers included
+DUMP_SEED = 0x5EEDB200
+
+
+def dump_outputs(out_dir, named_images):
+    """Write what the timed path returned to its caller in its last step: one (H, W, 3) float32 image per scene, as
+    DIR/<scene>.npy.  An image larger than its share of DUMP_BYTES is written as a fixed, seeded sample of its pixels
+    instead: DIR/<scene>.npy holds the (n, 3) sampled rows and DIR/<scene>_pixels.npy their flat pixel indices
+    (row * W + column, ascending, float64).  The sample depends on the image size only, so two builds run with the
+    same arguments are compared pixel for pixel."""
+    out_dir = Path(out_dir)
+    out_dir.mkdir(parents=True, exist_ok=True)
+    share = DUMP_BYTES // max(1, len(named_images))
+    for name, img in named_images:
+        img = np.ascontiguousarray(img)
+        if img.nbytes <= share:
+            np.save(out_dir / f"{name}.npy", img)
+            continue
+        rows = img.reshape(-1, img.shape[-1])
+        n = share // (rows.itemsize * rows.shape[1] + 8)
+        idx = np.sort(np.random.default_rng(DUMP_SEED).choice(rows.shape[0], size=n, replace=False))
+        np.save(out_dir / f"{name}.npy", rows[idx])
+        np.save(out_dir / f"{name}_pixels.npy", idx.astype(np.float64))
 
 
 def measured_peaks():
@@ -460,6 +498,8 @@ def run_ours(args):
     ms_total = float(ms.item())
     rays_all, launches_all = float(tot[0].item()), int(tot[1].item())
     census = {k: int(last[k]) for k in ("census_mismatch_pixels", "nan_pixels", "negative_pixels")} if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, [(spec.name, out[k].cpu().numpy()) for k, (spec, _, _) in enumerate(built)])
 
     # ---- end to end ---------------------------------------------------------------------------
     e2e_steps = args.e2e_steps or max(3, args.steps // 4)

@@ -11,8 +11,6 @@ from __future__ import annotations
 from dataclasses import dataclass
 from typing import Callable
 
-import os
-
 import numpy as np
 
 from .api import Axis, BvhHeuristic, Camera, Emission, Fresnel, Image, Material, Object, Scene, build_tables
@@ -211,14 +209,11 @@ def mesh_via_ply(vertices: np.ndarray, faces: np.ndarray, tag: str) -> np.ndarra
     import tempfile
     from pathlib import Path
     from . import mesh
-    d = Path(tempfile.gettempdir()) / "rayrs_b200_meshes"
-    d.mkdir(exist_ok=True)
-    path = d / f"{tag}_{os.getpid()}.ply"
-    mesh.write_ply(path, vertices, faces)
-    try:
+    # a private directory per call: a fixed shared one would belong to whichever user created it first
+    with tempfile.TemporaryDirectory(prefix="rayrs_b200_mesh_") as d:
+        path = Path(d) / f"{tag}.ply"
+        mesh.write_ply(path, vertices, faces)
         return mesh.load_ply_file(path)
-    finally:
-        path.unlink(missing_ok=True)
 
 
 COPPER = dict(color=(1, 1, 1), alpha=0.05, r0=(0.722, 0.451, 0.2))  # test_scenes.rs:154-159

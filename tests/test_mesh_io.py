@@ -95,12 +95,16 @@ def test_ply_writer_roundtrip(tmp_path, native_built, fmt):
         assert np.array_equal(np.frombuffer(body[: verts.size * 4], dtype=e + "f4").reshape(-1, 3), verts)
 
 
-def test_mesh_scene_goes_through_the_ply_loader(native_built):
+def test_mesh_scene_goes_through_the_ply_loader(native_built, tmp_path, monkeypatch):
+    import tempfile
+    monkeypatch.setattr(tempfile, "tempdir", str(tmp_path))
     spec = scenes.copper_torus(20, 10, 64, 48)
     verts, faces = scenes.torus_mesh(20, 10)
     tri_rows = spec.tables().objs
     tri_rows = tri_rows[tri_rows[:, 0] == 2][:, 3:12].reshape(-1, 3, 3)
     assert np.array_equal(tri_rows, scenes.mesh_triangles(verts, faces))
+    # the PLY file lived in a directory of its own, gone with it: nothing shared with other users is left behind
+    assert list(tmp_path.iterdir()) == []
 
 
 HEAD = "ply\nformat ascii 1.0\nelement vertex 1\nproperty float x\nproperty float y\nproperty float z\n"

@@ -3,23 +3,19 @@ it is held to what CAN be checked mechanically:
 
 * every `#[repr(C)]` struct and every `extern "C"` prototype of gpu.rs is the transcription of include/rayrs_b200.h:
   same fields in the same order with the same scalar types / array lengths / pointer-ness, same constants;
-* the patches are purely additive (main.rs too: the call goes in front of the rayon tile loop, which stays, compiled out)
-  and, where the reference sources are present (this container; not the GPU box), apply cleanly to them;
+* the patches are purely additive (main.rs too: the call goes in front of the rayon tile loop, which stays, compiled out),
+  well-formed for `patch -p1` (headers, hunk line counts, offsets), leave the patched files' delimiters balanced, and
+  put their context lines where the upstream lines this repository records (SURVEY.md) are;
 * everything gpu.rs uses from the patched modules (`BvhCursor`, `FlatGeom`, `FlatMaterial`, `Hittable::flatten`, ...) is
   defined by the patches.
 """
 import re
-import shutil
-import subprocess
 from pathlib import Path
-
-import pytest
 
 ROOT = Path(__file__).resolve().parents[1]
 HEADER = (ROOT / "include" / "rayrs_b200.h").read_text()
 GPU_RS = (ROOT / "rust" / "gpu.rs").read_text()
 PATCHES = sorted((ROOT / "rust" / "patches").glob("*.patch"))
-REFERENCE = Path("/root/reference")
 
 C_SCALAR = {"uint32_t": "u32", "int32_t": "i32", "uint64_t": "u64", "int64_t": "i64", "double": "f64", "float": "f32",
             "int": "c_int", "char": "c_char", "uint8_t": "u8", "size_t": "usize", "void": "c_void"}
@@ -163,6 +159,76 @@ def test_patches_only_add_lines():
         assert not removed, (p.name, removed[:3])  # main.rs.patch too: the CPU tile loop stays, compiled out
 
 
+# The upstream file each patch applies to.  The upstream sources are not part of this repository, so what follows holds
+# the patches to what `patch -p1` needs of them and to the few upstream lines this repository records (SURVEY.md).
+UPSTREAM = {"lib.rs.patch": "rayrs-lib/src/lib.rs", "geometry.rs.patch": "rayrs-lib/src/geometry.rs",
+            "material.rs.patch": "rayrs-lib/src/material.rs", "bvh.rs.patch": "rayrs-lib/src/bvh.rs",
+            "main.rs.patch": "rayrs/src/main.rs"}
+# rayrs/src/main.rs as SURVEY.md records it: the tile loop (`into_par_iter` over 16x16 tiles) spans lines 61-94,
+# between `Image::blocks` (57) and `Image::from_blocks` (101)
+MAIN_RS_LINES = {57: "Image::blocks(", 101: "Image::from_blocks("}
+TILE_LOOP = (61, 94)
+
+
+def _hunks(patch):
+    """[(old_start, old_len, new_start, new_len, [(old line number the line sits at or before, line)])] of a unified diff"""
+    lines = patch.read_text().splitlines()
+    out = []
+    for ln in lines[2:]:
+        m = re.fullmatch(r"@@ -(\d+),(\d+) \+(\d+),(\d+) @@.*", ln)
+        if m:
+            out.append(tuple(map(int, m.groups())) + ([],))
+            old = out[-1][0]
+            continue
+        assert out, (patch.name, ln)
+        out[-1][4].append((old, ln))
+        old += ln[:1] == " "
+    return out
+
+
+def test_patches_are_well_formed_unified_diffs():
+    """a/ and b/ headers naming the upstream file; hunk headers whose line counts are those of their bodies; hunks in
+    order without overlap, each new-file offset the old one shifted by the lines earlier hunks add."""
+    assert sorted(p.name for p in PATCHES) == sorted(UPSTREAM)
+    for p in PATCHES:
+        head = [ln.split("\t")[0] for ln in p.read_text().splitlines()[:2]]   # a timestamp may follow a tab
+        assert head == [f"--- a/{UPSTREAM[p.name]}", f"+++ b/{UPSTREAM[p.name]}"], (p.name, head)
+        hunks = _hunks(p)
+        assert hunks, p.name
+        shift, old_end = 0, 0
+        for o0, ol, n0, nl, body in hunks:
+            kinds = [ln[:1] for _, ln in body]
+            assert set(kinds) <= {" ", "+"}, (p.name, o0, set(kinds))
+            assert (ol, nl) == (kinds.count(" "), len(kinds)), (p.name, o0, ol, nl)
+            assert o0 > old_end and n0 == o0 + shift, (p.name, o0, n0, shift)
+            old_end, shift = o0 + ol - 1, shift + kinds.count("+")
+
+
+def test_patched_sources_keep_their_delimiters_balanced():
+    """The patches only add lines to sources that compile, so a patched file balances its braces and parentheses
+    exactly when the lines its patch adds do."""
+    for p in PATCHES:
+        text = _code_only("\n".join(ln[1:] for _, ln in sum((h[4] for h in _hunks(p)), []) if ln[:1] == "+"))
+        for a, b in ("{}", "()", "[]"):
+            assert text.count(a) == text.count(b), (p.name, a, text.count(a), text.count(b))
+
+
+def test_lib_rs_declares_the_module_and_main_rs_compiles_out_the_tile_loop():
+    lib = [ln[1:].strip() for _, ln in _hunks(ROOT / "rust" / "patches" / "lib.rs.patch")[0][4] if ln[:1] == "+"]
+    assert "pub mod gpu;" in lib
+    body = sum((h[4] for h in _hunks(ROOT / "rust" / "patches" / "main.rs.patch")), [])
+    # the context lines sit where the recorded upstream file has them
+    for at, text in MAIN_RS_LINES.items():
+        assert any(old == at and ln[:1] == " " and text in ln for old, ln in body), (at, text)
+    added = [(old, ln[1:].strip()) for old, ln in body if ln[:1] == "+"]
+    code = [ln for _, ln in added]
+    at = {ln: k for k, ln in enumerate(code)}
+    # the GPU call, then `#[cfg(any())] let image = {` (never true) in front of the tile loop, and its `};` after it
+    call = next(k for k, ln in enumerate(code) if "render_gpu(" in ln)
+    assert call < at["#[cfg(any())]"] == at["let image = {"] - 1 < at["};"]
+    assert added[at["let image = {"]][0] <= TILE_LOOP[0] and added[at["};"]][0] > TILE_LOOP[1]
+
+
 def test_gpu_rs_uses_only_what_the_patches_define():
     added = "\n".join(l[1:] for p in PATCHES for l in p.read_text().splitlines() if l.startswith("+") and not l.startswith("+++"))
     for item in ("BvhCursor", "FlatGeom", "FlatMaterial"):
@@ -177,35 +243,14 @@ def test_gpu_rs_uses_only_what_the_patches_define():
     assert used <= defined | {"len"}, (used, defined)
 
 
-@pytest.mark.skipif(not REFERENCE.exists() or shutil.which("patch") is None, reason="reference sources / patch(1) not present")
-def test_patches_apply_to_the_reference(tmp_path):
-    """on a scratch copy: /root/reference is read-only and nothing of it enters the repository"""
-    for sub in ("rayrs-lib/src", "rayrs/src"):
-        (tmp_path / sub).mkdir(parents=True)
-        for f in (REFERENCE / sub).glob("*.rs"):
-            shutil.copy(f, tmp_path / sub / f.name)
-    for p in PATCHES:
-        r = subprocess.run(["patch", "-p1", "--forward", "--batch", "-i", str(p)], cwd=tmp_path, stdout=subprocess.PIPE,
-                           stderr=subprocess.STDOUT, text=True)
-        assert r.returncode == 0, (p.name, r.stdout)
-        assert "FAILED" not in r.stdout and "fuzz" not in r.stdout, (p.name, r.stdout)
-    lib = (tmp_path / "rayrs-lib/src/lib.rs").read_text()
-    assert "pub mod gpu;" in lib
-    main = (tmp_path / "rayrs/src/main.rs").read_text()
-    # the call sits before the tile loop, which is compiled out (`#[cfg(any())]` is never true)
-    assert main.index("render_gpu(") < main.index("#[cfg(any())]") < main.index("into_par_iter")
-    # the patched sources still balance their braces (a cheap stand-in for the compiler that is not here)
-    for f in ("rayrs-lib/src/bvh.rs", "rayrs-lib/src/geometry.rs", "rayrs-lib/src/material.rs", "rayrs/src/main.rs"):
-        text = re.sub(r"//.*", "", (tmp_path / f).read_text())
-        text = re.sub(r'"(?:\\.|[^"\\])*"', '""', text)
-        text = re.sub(r"'(?:\\.|[^'\\])'", "' '", text)
-        assert text.count("{") == text.count("}"), f
-        assert text.count("(") == text.count(")"), f
+def _code_only(rust):
+    """Rust source without comments, string and char literals (a cheap stand-in for the compiler that is not here)"""
+    text = re.sub(r"//.*", "", rust)
+    text = re.sub(r'"(?:\\.|[^"\\])*"', '""', text)
+    return re.sub(r"'(?:\\.|[^'\\])'", "' '", text)
 
 
 def test_gpu_rs_balances_its_delimiters():
-    text = re.sub(r"//.*", "", GPU_RS)
-    text = re.sub(r'"(?:\\.|[^"\\])*"', '""', text)
-    text = re.sub(r"'(?:\\.|[^'\\])'", "' '", text)
+    text = _code_only(GPU_RS)
     for a, b in ("{}", "()", "[]"):
         assert text.count(a) == text.count(b), (a, text.count(a), text.count(b))
