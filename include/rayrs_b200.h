@@ -218,6 +218,16 @@ typedef struct RrsStats {
 #define RRS_FLAG_NO_L2_WINDOW 32u    /* this render: no L2 access-policy window over the node / primitive arrays (A/B) */
 #define RRS_FLAG_FORCE_PATHLOOP 16u /* small scenes (<= 8 primitives): use the register-resident path loop
                                        (k_pathloop) instead of the queued kernel (A/B measurements, tests) */
+#define RRS_FLAG_ENV_SAMPLING 64u   /* next-event estimation of the environment map: at every Lambertian or CookTorrance
+                                       vertex a direction is drawn from the map's importance-sampling table
+                                       (rrs_env_sample) and traced as a shadow ray, combined with the BSDF-sampled
+                                       continuation by multiple importance sampling (power heuristic).  The image
+                                       converges to the same mean as without the flag — the reference's estimator,
+                                       Russian roulette and quirks included — with less noise where the map's energy
+                                       is concentrated (a sun).  Other materials (Plastic, the glass / refract
+                                       variants, Reflect, NoReflect) and emission are shaded as without the flag.
+                                       Runs the fused queued kernel (RRS_FORM_WAVEFRONT; never the path loop; not with
+                                       RRS_FLAG_SPLIT_KERNELS) and doubles its ray queues. */
 
 typedef struct RrsScene RrsScene;
 
@@ -327,6 +337,15 @@ int rrs_material_evaluate_pdf(RrsScene* scene, uint32_t material, const RrsPrim*
 
 /* Scene::background (lib.rs:254-285) for a batch of directions (n x 3 doubles) -> n x 3 floats. */
 int rrs_background(RrsScene* scene, const double* dirs, size_t n, float* out);
+
+/* Parity probes of RRS_FLAG_ENV_SAMPLING's environment sampler.  rrs_env_sample: u = n x 2 uniforms in [0, 1) ->
+ * dir_pdf = n x 4 [unit direction xyz, solid-angle density] of the direction the render draws for them (each
+ * uniform's top 24 bits pick the cell of the table, the rest place the direction inside it).  Fails with
+ * RRS_ERR_INVALID on a black map.  rrs_env_pdf: dirs = n x 3 (need not be unit) -> pdf = n densities, exactly as the
+ * render evaluates them; 0 where the map is black.  The table is built once per scene by rrs_scene_create over the
+ * (w-1) x (h-1) cells between texel centres (4 bytes per cell + 8 per row of device memory). */
+int rrs_env_sample(RrsScene* scene, const double* u, size_t n, double* dir_pdf);
+int rrs_env_pdf(RrsScene* scene, const double* dirs, size_t n, double* pdf);
 
 /* The uniforms the device RNG hands to (pixel, sample, slot): 4 floats. */
 int rrs_rng_uniforms(RrsScene* scene, uint64_t seed, uint32_t pixel, uint32_t sample, uint32_t slot, float* out4);

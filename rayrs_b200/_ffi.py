@@ -23,6 +23,7 @@ RRS_FLAG_SPLIT_KERNELS = 4
 RRS_FLAG_FORCE_QUEUES = 8
 RRS_FLAG_FORCE_PATHLOOP = 16
 RRS_FLAG_NO_L2_WINDOW = 32
+RRS_FLAG_ENV_SAMPLING = 64
 RRS_SCENE_NO_BRUTE, RRS_SCENE_NO_BRUTE_BOX, RRS_SCENE_NO_L2_PERSIST = 1, 2, 4
 
 
@@ -116,6 +117,8 @@ CUDA_SYMBOLS = {
     "rrs_material_evaluate": (C.c_int, [C.c_void_p, C.c_uint32, C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p]),
     "rrs_material_evaluate_pdf": (C.c_int, [C.c_void_p, C.c_uint32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p]),
     "rrs_background": (C.c_int, [C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p]),
+    "rrs_env_sample": (C.c_int, [C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p]),
+    "rrs_env_pdf": (C.c_int, [C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p]),
     "rrs_rng_uniforms": (C.c_int, [C.c_void_p, C.c_uint64, C.c_uint32, C.c_uint32, C.c_uint32, C.c_void_p]),
     "rrs_bvh_build": (C.c_int, [C.c_void_p, C.c_uint32, C.c_uint32, C.c_uint32, C.c_int, C.c_void_p, C.c_void_p,
                                  C.POINTER(C.c_uint32), C.POINTER(C.c_double)]),

@@ -367,6 +367,23 @@ class Scene:
         _ffi.check(_ffi.cuda_lib().rrs_background(self.handle, d.ctypes.data, d.shape[0], out.ctypes.data))
         return out
 
+    def env_sample(self, u: np.ndarray) -> np.ndarray:
+        """rrs_env_sample: n x 2 uniforms in [0, 1) -> n x 4 (unit direction xyz, solid-angle density) as the
+        RRS_FLAG_ENV_SAMPLING render draws them."""
+        self._need_gpu()
+        uu = np.ascontiguousarray(u, dtype=np.float64).reshape(-1, 2)
+        out = np.zeros((uu.shape[0], 4), dtype=np.float64)
+        _ffi.check(_ffi.cuda_lib().rrs_env_sample(self.handle, uu.ctypes.data, uu.shape[0], out.ctypes.data))
+        return out
+
+    def env_pdf(self, dirs: np.ndarray) -> np.ndarray:
+        """rrs_env_pdf: the environment sampler's solid-angle density of n directions (n x 3)."""
+        self._need_gpu()
+        d = np.ascontiguousarray(dirs, dtype=np.float64).reshape(-1, 3)
+        out = np.zeros(d.shape[0], dtype=np.float64)
+        _ffi.check(_ffi.cuda_lib().rrs_env_pdf(self.handle, d.ctypes.data, d.shape[0], out.ctypes.data))
+        return out
+
     def rng_uniforms(self, seed: int, pixel: int, sample: int, slot: int) -> np.ndarray:
         self._need_gpu()
         out = np.zeros(4, dtype=np.float32)
@@ -390,6 +407,8 @@ class Scene:
 
 
 DEFAULT_SEED = 0x5EEDB200
+# render flag: next-event estimation of the environment map with MIS (include/rayrs_b200.h)
+RRS_FLAG_ENV_SAMPLING = _ffi.RRS_FLAG_ENV_SAMPLING
 
 
 def render_params(camera: Camera, spp: int, max_bounces: int, seed: int = DEFAULT_SEED, sample_offset: int = 0,

@@ -92,8 +92,79 @@ struct HostScene {
     std::vector<double4> sphere64;  // exact sphere parameters (see "sphere re-entry" in intersect.cuh)
     bool transmissive_sphere = false;
     std::vector<double> tri64;  // 9 doubles per primitive index, only when a triangle vertex is not exact in fp32
+    // environment sampling table (env.cuh): empty when the map is black; env_ok false when it cannot be tabulated
+    std::vector<float> env_marg, env_cond;
+    std::vector<float2> env_row;
+    bool env_ok = true;
     DScene d{};  // pointer members are filled per device
 };
+
+// Steps of a CDF over n cells of weights w (sum > 0), in units of 2^-24, the resolution of the device's uniforms:
+// proportional to w, at least one step for every positive cell, none for a zero cell, 2^24 in all.  Writes each
+// cell's start (exact in fp32).  False if the positive cells are too many for 2^24 steps.
+static bool quantize_cdf(const double* w, size_t n, double sum, float* start) {
+    const int64_t G = 1 << 24;
+    std::vector<int64_t> k(n);
+    int64_t tot = 0;
+    size_t big = 0;
+    for (size_t j = 0; j < n; ++j) {
+        k[j] = w[j] > 0. ? std::max<int64_t>(1, std::llround(w[j] / sum * (double)G)) : 0;
+        tot += k[j];
+        if (k[j] > k[big]) big = j;
+    }
+    k[big] += G - tot;  // rounding and the one-step minimum go to the largest cell
+    if (k[big] < 1) return false;
+    int64_t acc = 0;
+    for (size_t j = 0; j < n; ++j) {
+        start[j] = std::ldexp((float)acc, -24);
+        acc += k[j];
+    }
+    return true;
+}
+
+// The sampling table of RRS_FLAG_ENV_SAMPLING (env.cuh): per cell between texel centres the largest max(|r|,|g|,|b|)
+// of its 4 corners times its solid angle; the marginal CDF over rows and one conditional CDF per row.
+// 4 bytes per cell + 8 per row on the device (a 2048 x 1024 map: 8.4 MB).
+static void build_env_table(const std::vector<float4>& hdri, uint32_t w, uint32_t h, HostScene& out) {
+    const uint32_t cw = w - 1, ch = h - 1;
+    auto lum = [&](uint32_t i, uint32_t j) {
+        const float4 t = hdri[(size_t)i * w + j];
+        return std::max(std::fabs(t.x), std::max(std::fabs(t.y), std::fabs(t.z)));
+    };
+    std::vector<double> cell((size_t)cw * ch), rows(ch);
+    out.env_row.resize(ch);
+    const double dphi = 2. * M_PI / cw;
+    double total = 0.;
+    for (uint32_t i = 0; i < ch; ++i) {
+        const double t0 = M_PI * i / ch, t1 = M_PI * (i + 1) / ch;
+        const double dcos = 2. * std::sin(0.5 * (t0 + t1)) * std::sin(0.5 * (t1 - t0));  // cos t0 - cos t1
+        out.env_row[i] = make_float2((float)std::cos(t0), (float)dcos);
+        double r = 0.;
+        for (uint32_t j = 0; j < cw; ++j) {
+            const float m = std::max(std::max(lum(i, j), lum(i, j + 1)), std::max(lum(i + 1, j), lum(i + 1, j + 1)));
+            const double c = (double)m * dphi * dcos;
+            cell[(size_t)i * cw + j] = c;
+            r += c;
+        }
+        rows[i] = r;
+        total += r;
+    }
+    if (!std::isfinite(total)) {
+        out.env_ok = false;
+        return;
+    }
+    if (total == 0.) return;  // a black map: nothing to sample
+    out.env_marg.resize(ch);
+    out.env_cond.assign((size_t)cw * ch, 0.f);
+    bool ok = quantize_cdf(rows.data(), ch, total, out.env_marg.data());
+    for (uint32_t i = 0; i < ch && ok; ++i)
+        if (rows[i] > 0.) ok = quantize_cdf(cell.data() + (size_t)i * cw, cw, rows[i], out.env_cond.data() + (size_t)i * cw);
+    if (!ok) {
+        out.env_ok = false;
+        out.env_marg.clear();
+        out.env_cond.clear();
+    }
+}
 
 int validate_desc(const RrsSceneDesc* desc, std::string& err) {
     auto bad = [&](int code, const char* m) { err = m; return code; };
@@ -286,6 +357,7 @@ void convert_desc(const RrsSceneDesc* desc, HostScene& h) {
     h.hdri.resize(ntex);
     for (size_t i = 0; i < ntex; ++i)
         h.hdri[i] = make_float4(desc->hdri_rgb[3 * i], desc->hdri_rgb[3 * i + 1], desc->hdri_rgb[3 * i + 2], 0.f);
+    build_env_table(h.hdri, desc->hdri_width, desc->hdri_height, h);
     static_assert(sizeof(RrsNode) == 64, "RrsNode must be 64 bytes");
     static_assert(sizeof(RrsNodeF64) == 128, "RrsNodeF64 must be 128 bytes");
     {
@@ -442,6 +514,21 @@ int upload_scene(const RrsSceneDesc* desc, const HostScene& h, int device, RrsSc
     if (rc == RRS_OK) rc = upload(&s.mats, h.mats.data(), h.mats.size(), err);
     if (rc == RRS_OK) rc = upload(&s.emis, h.emis.data(), h.emis.size(), err);
     if (rc == RRS_OK) rc = upload(&s.hdri, h.hdri.data(), h.hdri.size(), err);
+    if (rc == RRS_OK && !h.env_marg.empty()) {
+        float* marg = nullptr;
+        float* cond = nullptr;
+        float2* row = nullptr;
+        rc = upload(&marg, h.env_marg.data(), h.env_marg.size(), err);
+        s.env.marg = marg;
+        if (rc == RRS_OK) rc = upload(&cond, h.env_cond.data(), h.env_cond.size(), err);
+        s.env.cond = cond;
+        if (rc == RRS_OK) rc = upload(&row, h.env_row.data(), h.env_row.size(), err);
+        s.env.row = row;
+    }
+    s.env.cw = desc->hdri_width - 1;
+    s.env.ch = desc->hdri_height - 1;
+    s.env.inv_dphi = (float)(s.env.cw / (2. * M_PI));
+    s.env_ok = h.env_ok;
     if (rc == RRS_OK && h.transmissive_sphere) rc = upload(&s.sphere64, h.sphere64.data(), h.sphere64.size(), err);
     if (rc == RRS_OK && !h.tri64.empty()) rc = upload(&s.tri64, h.tri64.data(), h.tri64.size(), err);
     if (rc == RRS_OK && desc->nodes_f64) {
@@ -518,6 +605,7 @@ void rrs_scene_destroy(RrsScene* scene) {
     cudaSetDevice(s.device);
     wf_free(&s);
     cudaFree(s.geom_blob); cudaFree(s.mats); cudaFree(s.emis); cudaFree(s.hdri);
+    cudaFree(const_cast<float*>(s.env.marg)); cudaFree(const_cast<float*>(s.env.cond)); cudaFree(const_cast<float2*>(s.env.row));
     cudaFree(s.prims_f64); cudaFree(s.nodes_f64); cudaFree(s.sphere64); cudaFree(s.tri64); cudaFree(s.accum); cudaFree(s.census); cudaFree(s.resolve_dev);
     if (s.resolve_pinned) cudaFreeHost(s.resolve_pinned);
     if (s.h_census) cudaFreeHost(s.h_census);
@@ -607,6 +695,20 @@ int rrs_background(RrsScene* scene, const double* dirs, size_t n, float* out) {
     if (!scene || (n && (!dirs || !out))) return fail(RRS_ERR_INVALID, "null argument");
     std::string err;
     int rc = wf_background(&scene->impl, dirs, n, out, err);
+    return rc == RRS_OK ? rc : fail(rc, err);
+}
+
+int rrs_env_sample(RrsScene* scene, const double* u, size_t n, double* dir_pdf) {
+    if (!scene || (n && (!u || !dir_pdf))) return fail(RRS_ERR_INVALID, "null argument");
+    std::string err;
+    int rc = wf_env_sample(&scene->impl, u, n, dir_pdf, err);
+    return rc == RRS_OK ? rc : fail(rc, err);
+}
+
+int rrs_env_pdf(RrsScene* scene, const double* dirs, size_t n, double* pdf) {
+    if (!scene || (n && (!dirs || !pdf))) return fail(RRS_ERR_INVALID, "null argument");
+    std::string err;
+    int rc = wf_env_pdf(&scene->impl, dirs, n, pdf, err);
     return rc == RRS_OK ? rc : fail(rc, err);
 }
 

@@ -437,12 +437,18 @@ __device__ __forceinline__ ScatterOut material_evaluate(const DMat& m, float3 n,
 // with probability ~0 in f64 but ~1e-4 in fp32, so the kernel always uses (1-fx, fx): that is
 // what the f64 reference computes for the real-valued x an fp32-integral x stands for.
 // Indices that the reference would panic on (theta == pi, phi == 2pi) are clamped.
-__device__ __forceinline__ float3 background(const DScene& sc, float3 dir) {
+// Texel coordinates of a direction (also the cell index of the environment's sampling table, env.cuh).
+__device__ __forceinline__ void background_coords(const DScene& sc, float3 dir, float& x, float& y) {
     dir = normalize3(dir);
     float phi = atan2f(dir.z, dir.x) + RRS_PI_F;
     float theta = acosf(fminf(1.f, fmaxf(-1.f, dir.y)));
-    float x = phi * (0.5f / RRS_PI_F) * (float)(sc.hdri_w - 1);
-    float y = theta * (1.0f / RRS_PI_F) * (float)(sc.hdri_h - 1);
+    x = phi * (0.5f / RRS_PI_F) * (float)(sc.hdri_w - 1);
+    y = theta * (1.0f / RRS_PI_F) * (float)(sc.hdri_h - 1);
+}
+
+__device__ __forceinline__ float3 background(const DScene& sc, float3 dir) {
+    float x, y;
+    background_coords(sc, dir, x, y);
     float xf = floorf(x), yf = floorf(y);
     float fx = x - xf, fy = y - yf;
     uint32_t j = (uint32_t)xf, i = (uint32_t)yf;

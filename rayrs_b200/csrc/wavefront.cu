@@ -186,13 +186,16 @@ __device__ __forceinline__ bool primary_ray(const RenderConst& rc, unsigned long
 // ---------------------------------------------------------------------------------------
 // generate: refill stripe b behind its survivors with new primary rays
 // ---------------------------------------------------------------------------------------
+// ENV (RRS_FLAG_ENV_SAMPLING): a path can have two rays in the next bounce (continuation + shadow ray), so the stripe
+// is filled to half its capacity; rays already in it (paths and shadow rays) count against that half.
+template <bool ENV = false>
 __device__ __forceinline__ void phase_generate(const RenderConst& rc, DCounters* __restrict__ c, const QueueSet& q, int cur,
                                                uint32_t* s_u32, unsigned long long* s_u64) {
     const uint32_t b = blockIdx.x;
     uint32_t* __restrict__ count = q.count + (size_t)cur * q.regions;
     const uint32_t n0 = count[b];
     if (threadIdx.x == 0) {
-        uint32_t need = q.region_cap - n0, got = 0;
+        uint32_t need = ENV ? (q.region_cap / 2u > n0 ? q.region_cap / 2u - n0 : 0u) : q.region_cap - n0, got = 0;
         unsigned long long base = 0;
         // claim `need` consecutive padded path indices (one global atomic per block per iteration)
         if (need && c->next_path < c->total_paths) {
@@ -434,9 +437,12 @@ struct NextRay {
     double p64[3];               // f64 hit point (transmissive spheres; written only when carry64)
 };
 
-template <bool SPH64, bool STAGED>
+// ENV: next-event estimation of the environment at a Lambertian or Cook-Torrance vertex (env.cuh).  *shadow gets the
+// shadow ray (its state carries what it adds if it escapes), *wcont the MIS weight of the continuation ray's escape.
+template <bool SPH64, bool STAGED, bool ENV = false>
 __device__ __forceinline__ NextRay shade_hit(const DScene& sc, const RenderConst& rc, float4* __restrict__ accum, float2 h,
-                                             float4 o4, float4 d4, float4 st, const double* o64_in) {
+                                             float4 o4, float4 d4, float4 st, const double* o64_in,
+                                             const DEnv* env = nullptr, NextRay* shadow = nullptr, float* wcont = nullptr) {
     NextRay nr;
     nr.alive = false;
     nr.carry64 = false;
@@ -472,6 +478,31 @@ __device__ __forceinline__ NextRay shade_hit(const DScene& sc, const RenderConst
     m.m1 = __ldg(mp + 1);
     m.m2 = __ldg(mp + 2);
     ScatterOut so = material_evaluate<STAGED>(m, nrm, view, u.x, u.y, u.z);
+    // NEE applies where the plain render traces a continuation at all, and not to a delta lobe (alpha^2 == 0 in fp32)
+    const bool nee = ENV && env->marg != nullptr && bounce + 1u < rc.max_bounces &&
+                     (mtag == RRS_MAT_LAMBERTIAN || (mtag == RRS_MAT_COOK_TORRANCE && m.m1.w > 0.f));
+    if (ENV) {
+        shadow->alive = false;
+        *wcont = 1.f;
+    }
+    if (nee) {
+        const float4 ue = rng_uniforms(rc.seed, pixel, sample, RRS_ENV_SLOT + bounce);
+        float3 l;
+        const float pe = env_sample(sc, *env, ue.x, ue.y, ue.z, ue.w, l);
+        float3 W;
+        const float pb = pe > 0.f ? nee_bsdf(m, mtag, nrm, view, l, W) : 0.f;
+        const float3 tw = mul3(thr, W);
+        const float p = fmaxf(fmaxf(tw.x, tw.y), tw.z);
+        if (pb > 0.f && p > 0.f) {
+            // the plain continuation survives Russian roulette with min(p, 1) and is divided by p
+            const float k = fminf(p, 1.f) / p * mis_cross(pe, pb);
+            const float3 bg = background(sc, l);
+            shadow->alive = true;
+            shadow->no = make_float4(pos.x, pos.y, pos.z, __uint_as_float(prim | RRS_SHADOW));
+            shadow->nd = make_float4(l.x, l.y, l.z, d4.w);
+            shadow->ns = make_float4(tw.x * bg.x * k, tw.y * bg.y * k, tw.z * bg.z * k, __uint_as_float(sb));
+        }
+    }
     bool finished = true;
     if (so.scatter) {
         // lib.rs:533-547
@@ -491,6 +522,12 @@ __device__ __forceinline__ NextRay shade_hit(const DScene& sc, const RenderConst
             no = make_float4(pos.x, pos.y, pos.z, __uint_as_float(carry64 ? (prim | RRS_ORG64) : prim));
             nd = make_float4(so.dir.x, so.dir.y, so.dir.z, d4.w);
             ns = make_float4(thr.x, thr.y, thr.z, __uint_as_float((sample << 8) | (bounce + 1u)));
+            if (nee) {
+                float3 W;
+                const float pb = nee_bsdf(m, mtag, nrm, view, so.dir, W);
+                const float pe = env_pdf(sc, *env, so.dir);
+                *wcont = pe > 0.f ? mis_power(pb, pe) : 1.f;
+            }
         }
     }
     if (finished) atomicAdd(accum + pixel, make_float4(0.f, 0.f, 0.f, 1.f));
@@ -511,10 +548,60 @@ __device__ __forceinline__ void shade_miss(const DScene& sc, float4* __restrict_
 // primitives, instead of in a separate extend phase — a fixed 8-primitive loop has nothing to gain from being
 // batched on its own, and fusing it drops the hit queue and the second read of every ray record (48 of ~190 bytes
 // of DRAM traffic per ray on the frosted-glass series, profiles/r01j_c3_frosted_metrics.csv).
-template <bool SPH64, bool INLINE_HIT, bool COUNT>
+// ENV (RRS_FLAG_ENV_SAMPLING): a shadow ray adds its state if it escapes and is dropped if it hits; a continuation
+// ray's escape is weighted by its MIS weight (env_miss); a shaded vertex may emit a shadow ray besides its
+// continuation (env_compact).
+__device__ __forceinline__ void env_miss(const DScene& sc, const DEnv& env, float4* __restrict__ accum, float4 o4, float4 d4,
+                                         float4 st, size_t slot) {
+    const uint32_t ow = __float_as_uint(o4.w);
+    if (ow != RRS_NO_PRIM && (ow & RRS_SHADOW)) {
+        atomicAdd(accum + __float_as_uint(d4.w), make_float4(st.x, st.y, st.z, 0.f));  // not a path end: .w stays
+        return;
+    }
+    const float w = ow == RRS_NO_PRIM ? 1.f : env.wmis[slot];  // camera rays: no other strategy
+    shade_miss(sc, accum, d4, make_float4(st.x * w, st.y * w, st.z * w, st.w));
+}
+
+__device__ __forceinline__ bool is_shadow_ray(float4 o4) {
+    const uint32_t ow = __float_as_uint(o4.w);
+    return ow != RRS_NO_PRIM && (ow & RRS_SHADOW);
+}
+
+// survivors and shadow rays of this warp take consecutive slots of the stripe (survivors first)
+template <bool SPH64>
+__device__ __forceinline__ void env_compact(const QueueSet& q, const DEnv& env, size_t ooff, uint32_t* s_out, const NextRay& nr,
+                                            const NextRay& sr, float wcont) {
+    const uint32_t lane = lane_id(), lt = (1u << lane) - 1u;
+    const uint32_t ba = __ballot_sync(0xFFFFFFFFu, nr.alive), bs = __ballot_sync(0xFFFFFFFFu, sr.alive);
+    if ((ba | bs) == 0u) return;
+    uint32_t obase = 0;
+    if (lane == 0) obase = atomicAdd(s_out, __popc(ba) + __popc(bs));
+    obase = __shfl_sync(0xFFFFFFFFu, obase, 0);
+    if (nr.alive) {
+        const uint32_t slot = obase + __popc(ba & lt);
+        RRS_CHECK(slot < q.region_cap);
+        stq(q.ray_o + ooff + slot, nr.no);
+        stq(q.ray_d + ooff + slot, nr.nd);
+        stq(q.state + ooff + slot, nr.ns);
+        stq(env.wmis + ooff + slot, wcont);
+        if (SPH64 && nr.carry64 && q.org64) {
+            double* o64 = q.org64 + 3 * (ooff + slot);
+            o64[0] = nr.p64[0]; o64[1] = nr.p64[1]; o64[2] = nr.p64[2];
+        }
+    }
+    if (sr.alive) {
+        const uint32_t slot = obase + __popc(ba) + __popc(bs & lt);
+        RRS_CHECK(slot < q.region_cap);
+        stq(q.ray_o + ooff + slot, sr.no);
+        stq(q.ray_d + ooff + slot, sr.nd);
+        stq(q.state + ooff + slot, sr.ns);
+    }
+}
+
+template <bool SPH64, bool INLINE_HIT, bool COUNT, bool ENV = false>
 __device__ __forceinline__ void phase_shade(const DScene& sc, const RenderConst& rc, DCounters* __restrict__ c,
                                             const QueueSet& q, int cur, float4* __restrict__ accum, uint32_t* s_cursor,
-                                            uint32_t* s_out, const DPrim* s_prims) {
+                                            uint32_t* s_out, const DPrim* s_prims, const DEnv* env = nullptr) {
     const uint32_t b = blockIdx.x;
     const uint32_t n = q.count[(size_t)cur * q.regions + b];
     const uint32_t lane = lane_id();
@@ -537,6 +624,9 @@ __device__ __forceinline__ void phase_shade(const DScene& sc, const RenderConst&
         NextRay nr;
         nr.alive = false;
         nr.carry64 = false;
+        NextRay sr;
+        sr.alive = false;
+        float wcont = 1.f;
         if (i < n) {
             float4 o4 = ldq(ray_o + i), d4 = ldq(ray_d + i), st = ldq(state + i);
             const double* o64 = (SPH64 && q.org64) ? q.org64 + 3 * (off + i) : nullptr;
@@ -548,11 +638,18 @@ __device__ __forceinline__ void phase_shade(const DScene& sc, const RenderConst&
             } else {
                 h = ldq(hits + i);
             }
-            if (__float_as_uint(h.y) == RRS_NO_PRIM) {
+            if (ENV) {
+                if (__float_as_uint(h.y) == RRS_NO_PRIM) env_miss(sc, *env, accum, o4, d4, st, off + i);
+                else if (!is_shadow_ray(o4)) nr = shade_hit<SPH64, true, true>(sc, rc, accum, h, o4, d4, st, o64, env, &sr, &wcont);
+            } else if (__float_as_uint(h.y) == RRS_NO_PRIM) {
                 shade_miss(sc, accum, d4, st);
             } else {
                 nr = shade_hit<SPH64, true>(sc, rc, accum, h, o4, d4, st, o64);
             }
+        }
+        if (ENV) {
+            env_compact<SPH64>(q, *env, ooff, s_out, nr, sr, wcont);
+            continue;
         }
         const bool alive = nr.alive;
         // queue compaction: survivors of this warp take consecutive slots of the stripe
@@ -604,10 +701,11 @@ __global__ void __launch_bounds__(kBlock, SPH64 ? RRS_BLOCKS_PER_SM_F64 : RRS_BL
 // write and one 48-byte read for the ~36 % of rays that continue, instead of generate-write / extend-read /
 // hit-write / shade-read (192 B of DRAM traffic per ray on the frosted-glass series, profiles/r01j_c3_frosted_*).
 // ---------------------------------------------------------------------------------------
-template <bool COUNT, bool SPH64>
+template <bool COUNT, bool SPH64, bool ENV = false>
 __device__ __forceinline__ bool small_scene_iteration(const DScene& sc, const RenderConst& rc, DCounters* __restrict__ c,
                                                       const QueueSet& q, int cur, float4* __restrict__ accum,
-                                                      const DPrim* s_prims, uint32_t* s_u32, unsigned long long* s_u64) {
+                                                      const DPrim* s_prims, uint32_t* s_u32, unsigned long long* s_u64,
+                                                      const DEnv* env = nullptr) {
     // s_u32: [0] new paths claimed, [1] rays traced, [2] work cursor, [3] append cursor; s_u64[0]: first new path index
     const uint32_t FULL = 0xFFFFFFFFu;
     const uint32_t b = blockIdx.x;
@@ -615,7 +713,8 @@ __device__ __forceinline__ bool small_scene_iteration(const DScene& sc, const Re
     const uint32_t lt_mask = (1u << lane) - 1u;
     const uint32_t n0 = q.count[(size_t)cur * q.regions + b];
     if (threadIdx.x == 0) {
-        uint32_t need = q.region_cap - n0, got = 0;
+        // ENV: fill to half the stripe, as phase_generate does
+        uint32_t need = ENV ? (q.region_cap / 2u > n0 ? q.region_cap / 2u - n0 : 0u) : q.region_cap - n0, got = 0;
         unsigned long long base = 0;
         if (need && c->next_path < c->total_paths) {  // one global atomic per block per iteration
             base = atomicAdd(&c->next_path, (unsigned long long)need);
@@ -671,14 +770,27 @@ __device__ __forceinline__ bool small_scene_iteration(const DScene& sc, const Re
                 st = make_float4(1.f, 1.f, 1.f, __uint_as_float(sample << 8));
             }
         }
+        NextRay sr;
+        sr.alive = false;
+        float wcont = 1.f;
         if (valid) {
             float2 h;
             uint32_t prim;
             closest_hit_brute<COUNT, SPH64>(sc, s_prims, xyz(o4), xyz(d4), __float_as_uint(o4.w), o64, h.x, prim, tcnt);
             h.y = __uint_as_float(prim);
             ++traced;
-            if (prim == RRS_NO_PRIM) shade_miss(sc, accum, d4, st);
-            else nr = shade_hit<SPH64, true>(sc, rc, accum, h, o4, d4, st, o64);
+            if (ENV) {
+                if (prim == RRS_NO_PRIM) env_miss(sc, *env, accum, o4, d4, st, off + i);  // (new paths: camera rays)
+                else if (!is_shadow_ray(o4)) nr = shade_hit<SPH64, true, true>(sc, rc, accum, h, o4, d4, st, o64, env, &sr, &wcont);
+            } else if (prim == RRS_NO_PRIM) {
+                shade_miss(sc, accum, d4, st);
+            } else {
+                nr = shade_hit<SPH64, true>(sc, rc, accum, h, o4, d4, st, o64);
+            }
+        }
+        if (ENV) {
+            env_compact<SPH64>(q, *env, ooff, &s_u32[3], nr, sr, wcont);
+            continue;
         }
         // queue compaction: survivors of this warp take consecutive slots of the stripe's other half
         const uint32_t ballot = __ballot_sync(FULL, nr.alive);
@@ -721,15 +833,15 @@ __device__ __forceinline__ bool small_scene_iteration(const DScene& sc, const Re
 // by the same SM while it is still in L2.  The three-kernel form above is kept (RRS_FLAG_SPLIT_KERNELS)
 // because it gives per-phase ncu evidence.
 // ---------------------------------------------------------------------------------------
-template <bool BRUTE, bool COUNT, bool SPH64>
+template <bool BRUTE, bool COUNT, bool SPH64, bool ENV>
 __device__ __forceinline__ bool wavefront_iteration(const DScene& sc, const RenderConst& rc, DCounters* __restrict__ c,
                                                     const QueueSet& q, int cur, float4* __restrict__ accum,
                                                     uint32_t* s_stack, const DPrim* s_prims, uint32_t* s_u32,
-                                                    unsigned long long* s_u64) {
+                                                    unsigned long long* s_u64, const DEnv* env) {
     // s_u64[1..3]: cycles spent in generate / extend / shade, s_u64[4]: iterations (thread 0 only)
     long long t0 = 0;
     if (threadIdx.x == 0) t0 = clock64();
-    phase_generate(rc, c, q, cur, s_u32, s_u64);
+    phase_generate<ENV>(rc, c, q, cur, s_u32, s_u64);
     __syncthreads();
     const uint32_t n = q.count[(size_t)cur * q.regions + blockIdx.x];
     if (threadIdx.x == 0) {
@@ -752,7 +864,7 @@ __device__ __forceinline__ bool wavefront_iteration(const DScene& sc, const Rend
         }
         __syncthreads();
     }
-    phase_shade<SPH64, BRUTE, COUNT>(sc, rc, c, q, cur, accum, &s_u32[2], &s_u32[3], s_prims);
+    phase_shade<SPH64, BRUTE, COUNT, ENV>(sc, rc, c, q, cur, accum, &s_u32[2], &s_u32[3], s_prims, env);
     __syncthreads();
     if (threadIdx.x == 0) {
         s_u64[3] += (unsigned long long)(clock64() - t0);
@@ -761,9 +873,9 @@ __device__ __forceinline__ bool wavefront_iteration(const DScene& sc, const Rend
     return true;
 }
 
-template <bool BRUTE, bool COUNT, bool SPH64>
-__global__ void __launch_bounds__(kBlock, SPH64 ? RRS_BLOCKS_PER_SM_F64 : RRS_BLOCKS_PER_SM) k_wavefront(DScene sc, RenderConst rc, DCounters* __restrict__ c,
-                                                                      QueueSet q, float4* __restrict__ accum) {
+template <bool BRUTE, bool COUNT, bool SPH64, bool ENV>
+__device__ __forceinline__ void wavefront_kernel(const DScene& sc, const RenderConst& rc, DCounters* __restrict__ c,
+                                                 const QueueSet& q, float4* __restrict__ accum, const DEnv* env) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
     uint32_t* s_stack = reinterpret_cast<uint32_t*>(smem_raw);
     __shared__ DPrim s_prims[RRS_BRUTE_MAX];
@@ -773,8 +885,8 @@ __global__ void __launch_bounds__(kBlock, SPH64 ? RRS_BLOCKS_PER_SM_F64 : RRS_BL
     stage_brute_prims(sc, s_prims);
     __syncthreads();
     for (int cur = 0;; cur ^= 1) {
-        const bool more = BRUTE ? small_scene_iteration<COUNT, SPH64>(sc, rc, c, q, cur, accum, s_prims, s_u32, s_u64)
-                                : wavefront_iteration<BRUTE, COUNT, SPH64>(sc, rc, c, q, cur, accum, s_stack, s_prims, s_u32, s_u64);
+        const bool more = BRUTE ? small_scene_iteration<COUNT, SPH64, ENV>(sc, rc, c, q, cur, accum, s_prims, s_u32, s_u64, env)
+                                : wavefront_iteration<BRUTE, COUNT, SPH64, ENV>(sc, rc, c, q, cur, accum, s_stack, s_prims, s_u32, s_u64, env);
         if (!more) break;
     }
     if (threadIdx.x == 0) {
@@ -783,6 +895,20 @@ __global__ void __launch_bounds__(kBlock, SPH64 ? RRS_BLOCKS_PER_SM_F64 : RRS_BL
         atomicAdd(&c->cyc_extend, s_u64[2]);
         atomicAdd(&c->cyc_shade, s_u64[3]);
     }
+}
+
+template <bool BRUTE, bool COUNT, bool SPH64>
+__global__ void __launch_bounds__(kBlock, SPH64 ? RRS_BLOCKS_PER_SM_F64 : RRS_BLOCKS_PER_SM) k_wavefront(DScene sc, RenderConst rc, DCounters* __restrict__ c,
+                                                                      QueueSet q, float4* __restrict__ accum) {
+    wavefront_kernel<BRUTE, COUNT, SPH64, false>(sc, rc, c, q, accum, nullptr);
+}
+
+// RRS_FLAG_ENV_SAMPLING: the same kernel with next-event estimation of the environment (separate instantiations, so
+// that the code of the default form does not change)
+template <bool BRUTE, bool COUNT, bool SPH64>
+__global__ void __launch_bounds__(kBlock, SPH64 ? RRS_BLOCKS_PER_SM_F64 : RRS_BLOCKS_PER_SM) k_wavefront_env(DScene sc, RenderConst rc, DCounters* __restrict__ c,
+                                                                          QueueSet q, float4* __restrict__ accum, DEnv env) {
+    wavefront_kernel<BRUTE, COUNT, SPH64, true>(sc, rc, c, q, accum, &env);
 }
 
 // ---------------------------------------------------------------------------------------
@@ -1016,6 +1142,21 @@ __global__ void k_background_probe(DScene sc, const float* __restrict__ dirs, ui
     out[3 * i] = c.x; out[3 * i + 1] = c.y; out[3 * i + 2] = c.z;
 }
 
+__global__ void k_env_sample_probe(DScene sc, DEnv env, const float4* __restrict__ u, uint32_t n, float4* __restrict__ out) {
+    uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    const float4 v = u[i];
+    float3 d;
+    const float pdf = env_sample(sc, env, v.x, v.y, v.z, v.w, d);
+    out[i] = make_float4(d.x, d.y, d.z, pdf);
+}
+
+__global__ void k_env_pdf_probe(DScene sc, DEnv env, const float* __restrict__ dirs, uint32_t n, float* __restrict__ out) {
+    uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    out[i] = env_pdf(sc, env, f3(dirs[3 * i], dirs[3 * i + 1], dirs[3 * i + 2]));
+}
+
 __global__ void k_rng_probe(uint64_t seed, uint32_t pixel, uint32_t sample, uint32_t slot, float* out) {
     float4 u = rng_uniforms(seed, pixel, sample, slot);
     out[0] = u.x; out[1] = u.y; out[2] = u.z; out[3] = u.w;
@@ -1029,7 +1170,8 @@ static size_t extend_smem_bytes(const DScene& d) {
 }
 
 static void free_queues(Wavefront& w) {
-    cudaFree(w.ray_o); cudaFree(w.ray_d); cudaFree(w.state); cudaFree(w.count); cudaFree(w.org64); cudaFree(w.hits);
+    cudaFree(w.ray_o); cudaFree(w.ray_d); cudaFree(w.state); cudaFree(w.count); cudaFree(w.org64); cudaFree(w.hits); cudaFree(w.wmis);
+    w.wmis = nullptr;
     w.ray_o = w.ray_d = w.state = nullptr;
     w.count = nullptr;
     w.org64 = nullptr;
@@ -1037,9 +1179,12 @@ static void free_queues(Wavefront& w) {
     w.capacity = 0;
 }
 
-static int ensure_wavefront(SceneImpl* s, uint32_t regions, uint32_t region_cap, std::string& err) {
+static int ensure_wavefront(SceneImpl* s, uint32_t regions, uint32_t region_cap, bool env, std::string& err) {
     Wavefront& w = s->wf;
-    if (w.regions == regions && w.region_cap == region_cap && w.capacity && w.counters) return RRS_OK;
+    if (w.regions == regions && w.region_cap == region_cap && w.capacity && w.counters) {
+        if (env && !w.wmis) RRS_CUDA_CHECK(cudaMalloc(&w.wmis, sizeof(float) * 2 * (size_t)w.capacity), err);
+        return RRS_OK;
+    }
     free_queues(w);
     const size_t cap = (size_t)regions * region_cap;
     RRS_CUDA_CHECK(cudaMalloc(&w.ray_o, sizeof(float4) * 2 * cap), err);
@@ -1048,6 +1193,7 @@ static int ensure_wavefront(SceneImpl* s, uint32_t regions, uint32_t region_cap,
     RRS_CUDA_CHECK(cudaMalloc(&w.count, sizeof(uint32_t) * 2 * regions), err);
     if (s->sphere64) RRS_CUDA_CHECK(cudaMalloc(&w.org64, sizeof(double) * 3 * 2 * cap), err);
     RRS_CUDA_CHECK(cudaMalloc(&w.hits, sizeof(float2) * cap), err);
+    if (env) RRS_CUDA_CHECK(cudaMalloc(&w.wmis, sizeof(float) * 2 * cap), err);
     if (!w.counters) RRS_CUDA_CHECK(cudaMalloc(&w.counters, sizeof(DCounters)), err);
     if (!w.h_counters) RRS_CUDA_CHECK(cudaMallocHost(&w.h_counters, sizeof(DCounters)), err);
     w.capacity = (uint32_t)cap;
@@ -1092,6 +1238,9 @@ int wf_render_accumulate(SceneImpl* s, const RrsCamera* cam, const RrsRenderPara
     if (p->max_bounces > 255) { err = "max_bounces > 255 not supported"; return RRS_ERR_INVALID; }
     if ((unsigned long long)p->sample_offset + p->spp > (1ull << 24)) { err = "sample index exceeds 2^24"; return RRS_ERR_INVALID; }
     if ((unsigned long long)p->width * p->height > 0xFFFFFFFFull) { err = "image too large"; return RRS_ERR_INVALID; }
+    const bool env = (p->flags & RRS_FLAG_ENV_SAMPLING) != 0;
+    if (env && (p->flags & RRS_FLAG_SPLIT_KERNELS)) { err = "RRS_FLAG_ENV_SAMPLING runs in the fused kernel only (not with RRS_FLAG_SPLIT_KERNELS)"; return RRS_ERR_INVALID; }
+    if (env && !s->env_ok) { err = "the environment map cannot be tabulated for sampling (non-finite texels)"; return RRS_ERR_INVALID; }
     RRS_CUDA_CHECK(cudaSetDevice(s->device), err);
     wf_finish_stats(s);  // a scene's queues and counters serve one render at a time
     // ---- launch geometry: every kernel runs `regions` blocks, block b owns queue stripe b ----
@@ -1121,14 +1270,21 @@ int wf_render_accumulate(SceneImpl* s, const RrsCamera* cam, const RrsRenderPara
                                      k_wavefront<true, false, false>,  k_wavefront<true, false, true>,
                                      k_wavefront<true, true, false>,   k_wavefront<true, true, true>};
     FusedFn fused_fn = table[sel];
-    RRS_CUDA_CHECK(cudaFuncSetAttribute(fused_fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem), err);
+    typedef void (*EnvFusedFn)(DScene, RenderConst, DCounters*, QueueSet, float4*, DEnv);
+    static const EnvFusedFn env_table[8] = {k_wavefront_env<false, false, false>, k_wavefront_env<false, false, true>,
+                                            k_wavefront_env<false, true, false>,  k_wavefront_env<false, true, true>,
+                                            k_wavefront_env<true, false, false>,  k_wavefront_env<true, false, true>,
+                                            k_wavefront_env<true, true, false>,   k_wavefront_env<true, true, true>};
+    EnvFusedFn env_fn = env_table[sel];
+    const void* fused_kernel = env ? (const void*)env_fn : (const void*)fused_fn;
+    RRS_CUDA_CHECK(cudaFuncSetAttribute(fused_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem), err);
     auto generate_fn = k_generate;
     RRS_CUDA_CHECK(cudaFuncSetAttribute(extend_fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem), err);
     int occ_ext = 0, occ_shade = 0;
     RRS_CUDA_CHECK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ_ext, extend_fn, kBlock, smem), err);
     RRS_CUDA_CHECK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ_shade, shade_fn, kBlock, 0), err);
     int occ_fused = 0;
-    RRS_CUDA_CHECK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ_fused, fused_fn, kBlock, smem), err);
+    RRS_CUDA_CHECK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ_fused, fused_kernel, kBlock, smem), err);
     if (occ_ext < 1 || occ_shade < 1 || occ_fused < 1) { err = "kernel does not fit on an SM (traversal stack too deep)"; return RRS_ERR_TOO_DEEP; }
     if (!(p->flags & RRS_FLAG_SPLIT_KERNELS)) occ_ext = occ_shade = occ_fused;
     // one wave of the most register-hungry kernel: all stripes are resident at once
@@ -1137,7 +1293,9 @@ int wf_render_accumulate(SceneImpl* s, const RrsCamera* cam, const RrsRenderPara
     // configuration 4 +1.5 % over 4M; 16M / 32M within 1 % of 8M — profiles/ab_logs/queue_r02x.log)
     uint32_t want = p->queue_capacity ? p->queue_capacity : (brute ? (1u << 22) : (1u << 23));
     uint32_t region_cap = std::max(32u, ((want + regions - 1) / regions + 31u) & ~31u);
-    int rc_ = ensure_wavefront(s, regions, region_cap, err);
+    // environment sampling: as many paths in flight, and room for a shadow ray beside each continuation
+    if (env) region_cap *= 2u;
+    int rc_ = ensure_wavefront(s, regions, region_cap, env, err);
     if (rc_ != RRS_OK) return rc_;
     Wavefront& w = s->wf;
     RRS_CUDA_CHECK(cudaMemsetAsync(w.count, 0, sizeof(uint32_t) * 2 * regions, stream), err);
@@ -1247,12 +1405,18 @@ int wf_render_accumulate(SceneImpl* s, const RrsCamera* cam, const RrsRenderPara
     // fast or faster on every small scene (plastic series +5 %, sweep_pl_vs_q.log) — compaction gives it full warps
     // every iteration — so the path loop is an option (RRS_FLAG_FORCE_PATHLOOP), not the default.
     const bool want_pathloop = (p->flags & RRS_FLAG_FORCE_PATHLOOP) != 0;
-    const bool pathloop = !split && brute && want_pathloop && !(p->flags & RRS_FLAG_FORCE_QUEUES);
+    const bool pathloop = !split && brute && want_pathloop && !(p->flags & RRS_FLAG_FORCE_QUEUES) && !env;
     if (pathloop) {
         // small scene: register-resident paths, no queues (k_pathloop)
         int occ_path = 0;
         RRS_CUDA_CHECK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ_path, path_fn, kBlock, 0), err);
         path_fn<<<(uint32_t)s->num_sms * (uint32_t)std::max(occ_path, 1), kBlock, 0, stream>>>(s->d, rc, w.counters, d_accum);
+        launches = 1;
+        RRS_CUDA_CHECK(cudaGetLastError(), err);
+    } else if (env) {
+        DEnv e = s->env;
+        e.wmis = w.wmis;
+        env_fn<<<regions, kBlock, smem, stream>>>(s->d, rc, w.counters, q, d_accum, e);
         launches = 1;
         RRS_CUDA_CHECK(cudaGetLastError(), err);
     } else if (!split) {
@@ -1495,6 +1659,57 @@ int wf_background(SceneImpl* s, const double* dirs, size_t n, float* out, std::s
     k_background_probe<<<(unsigned)((n + 127) / 128), 128>>>(s->d, d_d, (uint32_t)n, d_out);
     RRS_CUDA_CHECK(cudaGetLastError(), err);
     RRS_CUDA_CHECK(cudaMemcpy(out, d_out, sizeof(float) * 3 * n, cudaMemcpyDeviceToHost), err);
+    return RRS_OK;
+}
+
+int wf_env_sample(SceneImpl* s, const double* u, size_t n, double* dir_pdf, std::string& err) {
+    if (!s->env_ok) { err = "the environment map cannot be tabulated for sampling (non-finite texels)"; return RRS_ERR_INVALID; }
+    if (!s->env.marg) { err = "the environment map is black: nothing to sample"; return RRS_ERR_INVALID; }
+    RRS_CUDA_CHECK(cudaSetDevice(s->device), err);
+    if (n == 0) return RRS_OK;
+    if (n > 0x7FFFFFFFull) { err = "too many samples"; return RRS_ERR_INVALID; }
+    // each uniform in [0, 1) as the device draws it: 24 bits that pick the cell + 24 more (hi, lo: env_sample)
+    std::vector<float4> hu(n);
+    auto split = [](double v, float& hi, float& lo) {
+        const double x = std::ldexp(std::min(std::max(v, 0.), 1.), 24);
+        const double f = std::min(std::floor(x), 16777215.);
+        hi = (float)std::ldexp(f, -24);
+        lo = (float)std::min(x - f, 1.);
+    };
+    for (size_t i = 0; i < n; ++i) {
+        split(u[2 * i], hu[i].x, hu[i].z);
+        split(u[2 * i + 1], hu[i].y, hu[i].w);
+    }
+    DevBuf<float4> d_u, d_out;
+    RRS_CUDA_CHECK(d_u.alloc(n), err);
+    RRS_CUDA_CHECK(d_out.alloc(n), err);
+    RRS_CUDA_CHECK(cudaMemcpy(d_u, hu.data(), sizeof(float4) * n, cudaMemcpyHostToDevice), err);
+    k_env_sample_probe<<<(unsigned)((n + 127) / 128), 128>>>(s->d, s->env, d_u, (uint32_t)n, d_out);
+    RRS_CUDA_CHECK(cudaGetLastError(), err);
+    std::vector<float4> ho(n);
+    RRS_CUDA_CHECK(cudaMemcpy(ho.data(), d_out, sizeof(float4) * n, cudaMemcpyDeviceToHost), err);
+    for (size_t i = 0; i < n; ++i) {
+        dir_pdf[4 * i] = ho[i].x; dir_pdf[4 * i + 1] = ho[i].y; dir_pdf[4 * i + 2] = ho[i].z; dir_pdf[4 * i + 3] = ho[i].w;
+    }
+    return RRS_OK;
+}
+
+int wf_env_pdf(SceneImpl* s, const double* dirs, size_t n, double* pdf, std::string& err) {
+    if (!s->env_ok) { err = "the environment map cannot be tabulated for sampling (non-finite texels)"; return RRS_ERR_INVALID; }
+    RRS_CUDA_CHECK(cudaSetDevice(s->device), err);
+    if (n == 0) return RRS_OK;
+    if (n > 0x7FFFFFFFull) { err = "too many directions"; return RRS_ERR_INVALID; }
+    std::vector<float> hd(3 * n);
+    for (size_t i = 0; i < 3 * n; ++i) hd[i] = (float)dirs[i];
+    DevBuf<float> d_d, d_out;
+    RRS_CUDA_CHECK(d_d.alloc(3 * n), err);
+    RRS_CUDA_CHECK(d_out.alloc(n), err);
+    RRS_CUDA_CHECK(cudaMemcpy(d_d, hd.data(), sizeof(float) * 3 * n, cudaMemcpyHostToDevice), err);
+    k_env_pdf_probe<<<(unsigned)((n + 127) / 128), 128>>>(s->d, s->env, d_d, (uint32_t)n, d_out);
+    RRS_CUDA_CHECK(cudaGetLastError(), err);
+    std::vector<float> ho(n);
+    RRS_CUDA_CHECK(cudaMemcpy(ho.data(), d_out, sizeof(float) * n, cudaMemcpyDeviceToHost), err);
+    for (size_t i = 0; i < n; ++i) pdf[i] = ho[i];
     return RRS_OK;
 }
 

@@ -7,6 +7,7 @@
 #include <vector>
 
 #include "device_types.cuh"
+#include "env.cuh"
 
 namespace rrs {
 
@@ -52,6 +53,7 @@ struct Wavefront {
     float4* state = nullptr;    // [2][capacity] throughput rgb, sample << 8 | bounce
     float2* hits = nullptr;     // [capacity]    t, primitive
     double* org64 = nullptr;    // [2][capacity][3] f64 hit points of rays spawned on transmissive spheres
+    float* wmis = nullptr;      // [2][capacity] MIS weight of continuation rays (RRS_FLAG_ENV_SAMPLING renders only)
     DCounters* counters = nullptr;
     DCounters* h_counters = nullptr;  // pinned
 };
@@ -73,6 +75,10 @@ struct SceneImpl {
     RrsNodeF64* nodes_f64 = nullptr;
     double4* sphere64 = nullptr;
     double* tri64 = nullptr;
+    // environment sampling table (env.cuh; env.wmis is set per render).  env_ok: the table exists, or the map is black
+    // and there is nothing to sample (env.marg == nullptr); false when the map cannot be tabulated
+    DEnv env{};
+    bool env_ok = false;
     uint32_t n_prims = 0, n_nodes = 0;
     uint32_t max_depth = 0;
     double tmin = 0, tmax = 0;
@@ -115,6 +121,8 @@ int wf_material_evaluate(SceneImpl* s, uint32_t material, const double* nv, cons
 int wf_background(SceneImpl* s, const double* dirs, size_t n, float* out, std::string& err);
 int wf_rng_uniforms(SceneImpl* s, uint64_t seed, uint32_t pixel, uint32_t sample, uint32_t slot, float* out4,
                     std::string& err);
+int wf_env_sample(SceneImpl* s, const double* u, size_t n, double* dir_pdf, std::string& err);
+int wf_env_pdf(SceneImpl* s, const double* dirs, size_t n, double* pdf, std::string& err);
 void wf_finish_stats(SceneImpl* s);  // waits for the last render of this scene and completes s->stats
 void wf_free(SceneImpl* s);
 // verify_f64.cu

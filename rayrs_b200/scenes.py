@@ -74,6 +74,14 @@ def synthetic_hdri(width: int = 2048, height: int = 1024) -> Image:
     return Image(width, height, np.clip(img, 0.0, 3.0))
 
 
+def sun_hdri(width: int = 128, height: int = 64, sky: float = 1.0, sun: float = 2000.0) -> Image:
+    """Unclipped environment for environment sampling (RRS_FLAG_ENV_SAMPLING): a uniform sky and a 3 x 3-texel sun
+    `sun / sky` times brighter, high in the sky — most of the light in a small part of the map."""
+    px = np.full((height, width, 3), float(sky))
+    px[height // 4 - 1:height // 4 + 2, width // 3 - 1:width // 3 + 2] = (sun, 0.95 * sun, 0.85 * sun)
+    return Image(width, height, px)
+
+
 # ---------------------------------------------------------------------------------------
 # test_scenes.rs
 # ---------------------------------------------------------------------------------------
@@ -291,6 +299,17 @@ class Config:
     height: int
     spp: int
     max_bounces: int
+
+
+def sun_spheres(width_px=64, height_px=48) -> SceneSpec:
+    """A Lambertian and a rough metallic Cook-Torrance sphere (alpha 0.3) on the rough metallic floor, for sun_hdri."""
+    w, h = film(width_px, height_px)
+    objects = [_floor(),
+               Object.sphere(1.0, (-1.2, 1.0, 0.0), Material.lambertian_diffuse((0.8, 0.7, 0.6)), Emission.Dark()),
+               Object.sphere(1.0, (1.2, 1.0, 0.0), Material.cook_torrance((0.9, 0.9, 0.9), 0.3, Fresnel.schlick_metallic((0.9, 0.6, 0.3))),
+                             Emission.Dark())]
+    cam = dict(origin=(0.0, 4.0, 9.0), up=(0.0, 1.0, 0.0), lookat=(0.0, 1.0, 0.0), fov=50.0, width=w, height=h, ppi=PPI)
+    return SceneSpec("sun_spheres", cam, objects, BvhHeuristic.Sah(1000), max_bounces=16)
 
 
 def _c1():

@@ -37,6 +37,8 @@ use crate::{Camera, Object, Scene};
 pub const RRS_ABI_VERSION: u32 = 2;
 pub const RRS_REF_LEAF: u32 = 0x8000_0000;
 pub const RRS_REF_EMPTY: u32 = 0xFFFF_FFFF;
+/// RrsRenderParams.flags: next-event estimation of the environment map with MIS (include/rayrs_b200.h)
+pub const RRS_FLAG_ENV_SAMPLING: u32 = 64;
 
 #[repr(C)]
 #[derive(Clone, Copy, Default)]
@@ -189,6 +191,11 @@ extern "C" {
         cuda_streams: *const *mut c_void,
     ) -> c_int;
     fn rrs_stats(scene: *mut RrsScene, out: *mut RrsStats) -> c_int;
+    // parity probes of the environment sampler (RRS_FLAG_ENV_SAMPLING)
+    #[allow(dead_code)]
+    fn rrs_env_sample(scene: *mut RrsScene, u: *const f64, n: usize, dir_pdf: *mut f64) -> c_int;
+    #[allow(dead_code)]
+    fn rrs_env_pdf(scene: *mut RrsScene, dirs: *const f64, n: usize, pdf: *mut f64) -> c_int;
     fn rrs_last_error() -> *const c_char;
     fn rrs_device_count() -> c_int;
 }
