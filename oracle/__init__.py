@@ -43,6 +43,14 @@ def lib() -> C.CDLL:
         L.orc_camera_new.argtypes = [vp, vp, vp, dbl, dbl, dbl, u32, vp]
         L.orc_primary_rays.argtypes = [vp, u32, u32, vp, vp, vp, u64, u64, i32, vp]
         L.orc_render.argtypes = [vp, vp, u32, u32, u32, u32, u32, u64, i32, i32, vp, vp]
+        L.orc_render_env.restype = i32
+        L.orc_render_env.argtypes = [vp, vp, u32, u32, u32, u32, u32, u64, i32, i32, vp, vp]
+        L.orc_env_table.restype = i32
+        L.orc_env_table.argtypes = [vp, vp, vp, vp]
+        L.orc_env_sample.restype = i32
+        L.orc_env_sample.argtypes = [vp, vp, u64, vp]
+        L.orc_env_pdf.restype = i32
+        L.orc_env_pdf.argtypes = [vp, vp, u64, vp]
         L.orc_material_evaluate.argtypes = [vp, vp, vp, u64, vp]
         L.orc_material_evaluate_pdf.argtypes = [vp, vp, vp, vp, u64, vp]
         L.orc_hittable_area_sample.argtypes = [vp, vp, vp]
@@ -137,15 +145,55 @@ class OracleScene:
                                         tc.ctypes.data, nthreads or hardware_threads())
         return st.astype(bool), tc
 
-    def render(self, cam17, W, H, spp, max_bounces=50, seed=0x5EEDB200, sample_offset=0, rng_mode=RNG_MATCHED, nthreads=0):
+    def render(self, cam17, W, H, spp, max_bounces=50, seed=0x5EEDB200, sample_offset=0, rng_mode=RNG_MATCHED, nthreads=0,
+               env=False):
+        """env=True: with the GPU backend's environment sampling (RRS_FLAG_ENV_SAMPLING); the stats then also hold
+        shadow_rays (counted in rays as well).  Raises ValueError for a map the flag refuses (non-finite texels)."""
         out = np.zeros((H, W, 3), dtype=np.float64)
-        stats = np.zeros(7, dtype=np.uint64)
+        stats = np.zeros(8, dtype=np.uint64)
         c = _d(cam17)
-        lib().orc_render(self._p, c.ctypes.data, W, H, spp, sample_offset, max_bounces, seed, rng_mode,
-                         nthreads or hardware_threads(), out.ctypes.data, stats.ctypes.data)
-        return out, dict(rays=int(stats[0]), scatters=int(stats[1]), nan_pixels=int(stats[2]),
-                         negative_pixels=int(stats[3]), seconds=float(stats[4]) * 1e-6,
-                         reentry_total=int(stats[5]), reentry_lost=int(stats[6]))
+        args = (self._p, c.ctypes.data, W, H, spp, sample_offset, max_bounces, seed, rng_mode,
+                nthreads or hardware_threads(), out.ctypes.data, stats.ctypes.data)
+        if env:
+            if lib().orc_render_env(*args) != 0:
+                raise ValueError("the environment map cannot be tabulated for sampling (non-finite texels)")
+        else:
+            lib().orc_render(*args)
+        st = dict(rays=int(stats[0]), scatters=int(stats[1]), nan_pixels=int(stats[2]),
+                  negative_pixels=int(stats[3]), seconds=float(stats[4]) * 1e-6,
+                  reentry_total=int(stats[5]), reentry_lost=int(stats[6]))
+        if env:
+            st["shadow_rays"] = int(stats[7])
+        return out, st
+
+    def env_table(self):
+        """The environment-sampling table (rayrs_b200/csrc/api.cu build_env_table): dict(marg (ch,), cond (ch, cw),
+        row (ch, 2)) as float32, None for a black map; ValueError for a map with non-finite texels."""
+        hh, hw = self.hdri.shape[:2]
+        marg = np.zeros(hh - 1, dtype=np.float32)
+        cond = np.zeros((hh - 1, hw - 1), dtype=np.float32)
+        row = np.zeros((hh - 1, 2), dtype=np.float32)
+        rc = lib().orc_env_table(self._p, marg.ctypes.data, cond.ctypes.data, row.ctypes.data)
+        if rc < 0:
+            raise ValueError("the environment map cannot be tabulated for sampling (non-finite texels)")
+        return dict(marg=marg, cond=cond, row=row) if rc == 1 else None
+
+    def env_sample(self, u):
+        """rrs_env_sample's inputs (n x 2 uniforms in [0, 1)) -> n x 6: direction xyz, density of the drawn cell,
+        cell row, cell column."""
+        uu = _d(u).reshape(-1, 2)
+        out = np.zeros((uu.shape[0], 6))
+        if lib().orc_env_sample(self._p, uu.ctypes.data, uu.shape[0], out.ctypes.data) != 0:
+            raise ValueError("nothing to sample: the map is black or has non-finite texels")
+        return out
+
+    def env_pdf(self, dirs):
+        """rrs_env_pdf: the density of n directions (n x 3) in the cell Scene::background reads them from."""
+        d = _d(dirs).reshape(-1, 3)
+        out = np.zeros(d.shape[0])
+        if lib().orc_env_pdf(self._p, d.ctypes.data, d.shape[0], out.ctypes.data) != 0:
+            raise ValueError("the environment map cannot be tabulated for sampling (non-finite texels)")
+        return out
 
     def background(self, dirs):
         d = _d(dirs).reshape(-1, 3)

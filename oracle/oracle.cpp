@@ -31,6 +31,11 @@
 // counter-based Philox4x32-7 stream keyed by (seed; pixel, sample, slot) so that
 // results are reproducible and can be sample-matched with the GPU backend.
 //
+// One addition that is not in the reference: the GPU backend's environment sampling (RRS_FLAG_ENV_SAMPLING), restated
+// from rayrs_b200/csrc/api.cu build_env_table and env.cuh / wavefront.cu (EnvTable, env_sample, nee_bsdf, radiance with
+// env; orc_render_env, orc_env_table, orc_env_sample, orc_env_pdf) so that ENV images can be sample-matched too.
+// orc_render and radiance without it are unchanged.
+//
 // Build: see oracle/Makefile (g++ -O3 -ffp-contract=off: Rust never contracts a*b+c).
 
 #include <algorithm>
@@ -967,8 +972,180 @@ static inline Ray camera_primary_ray(const Camera& c, size_t i, size_t j, double
     return Ray{c.origin, c.z + x * c.e_x + y * c.e_y};
 }
 
+// ------------------------------------------------------------------------------------
+// Environment importance sampling (the GPU backend's RRS_FLAG_ENV_SAMPLING; not part of the reference).  Restates
+// rayrs_b200/csrc/api.cu build_env_table / quantize_cdf (the table, bit for bit: the same f64 arithmetic, fp32
+// arrays) and env.cuh (sampler, density, nee_bsdf, MIS weights) in f64.
+// ------------------------------------------------------------------------------------
+struct EnvTable {
+    bool ok = true;                  // false: a non-finite texel (the render refuses the flag)
+    uint32_t cw = 0, ch = 0;         // cells: hdri_w - 1, hdri_h - 1
+    std::vector<float> marg, cond;   // CDF starts, multiples of 2^-24; marg empty: a black map
+    std::vector<float> cos0, dcos;   // per row: cos theta at the top edge, cos top - cos bottom
+    float inv_dphi = 0.f;            // cw / 2pi
+};
+
+static bool quantize_cdf(const double* w, size_t n, double sum, float* start) {
+    const int64_t G = 1 << 24;
+    std::vector<int64_t> k(n);
+    int64_t tot = 0;
+    size_t big = 0;
+    for (size_t j = 0; j < n; ++j) {
+        k[j] = w[j] > 0. ? std::max<int64_t>(1, std::llround(w[j] / sum * (double)G)) : 0;
+        tot += k[j];
+        if (k[j] > k[big]) big = j;
+    }
+    k[big] += G - tot;
+    if (k[big] < 1) return false;
+    int64_t acc = 0;
+    for (size_t j = 0; j < n; ++j) {
+        start[j] = std::ldexp((float)acc, -24);
+        acc += k[j];
+    }
+    return true;
+}
+
+static void build_env_table(const std::vector<V3>& hdri, size_t w, size_t h, EnvTable& out) {
+    out = EnvTable();
+    const uint32_t cw = (uint32_t)w - 1, ch = (uint32_t)h - 1;
+    out.cw = cw;
+    out.ch = ch;
+    out.inv_dphi = (float)(cw / (2. * PI));
+    for (const V3& t : hdri)
+        if (!std::isfinite((float)t.x) || !std::isfinite((float)t.y) || !std::isfinite((float)t.z)) {
+            out.ok = false;
+            return;
+        }
+    auto lum = [&](uint32_t i, uint32_t j) {
+        const V3& t = hdri[(size_t)i * w + j];
+        return std::max(std::fabs((float)t.x), std::max(std::fabs((float)t.y), std::fabs((float)t.z)));
+    };
+    std::vector<double> cell((size_t)cw * ch), rows(ch);
+    out.cos0.resize(ch);
+    out.dcos.resize(ch);
+    const double dphi = 2. * PI / cw;
+    double total = 0.;
+    for (uint32_t i = 0; i < ch; ++i) {
+        const double t0 = PI * i / ch, t1 = PI * (i + 1) / ch;
+        const double dcos = 2. * std::sin(0.5 * (t0 + t1)) * std::sin(0.5 * (t1 - t0));
+        out.cos0[i] = (float)std::cos(t0);
+        out.dcos[i] = (float)dcos;
+        double r = 0.;
+        for (uint32_t j = 0; j < cw; ++j) {
+            const float m = std::max(std::max(lum(i, j), lum(i, j + 1)), std::max(lum(i + 1, j), lum(i + 1, j + 1)));
+            const double c = (double)m * dphi * dcos;
+            cell[(size_t)i * cw + j] = c;
+            r += c;
+        }
+        rows[i] = r;
+        total += r;
+    }
+    if (!std::isfinite(total)) { out.ok = false; return; }
+    if (total == 0.) return;
+    out.marg.resize(ch);
+    out.cond.assign((size_t)cw * ch, 0.f);
+    bool ok = quantize_cdf(rows.data(), ch, total, out.marg.data());
+    for (uint32_t i = 0; i < ch && ok; ++i)
+        if (rows[i] > 0.) ok = quantize_cdf(cell.data() + (size_t)i * cw, cw, rows[i], out.cond.data() + (size_t)i * cw);
+    if (!ok) {
+        out.ok = false;
+        out.marg.clear();
+        out.cond.clear();
+    }
+}
+
+// largest k < n with a[k] <= u; the step of cell k (exact: multiples of 2^-24)
+static inline uint32_t cdf_find(const float* a, uint32_t n, double u) {
+    return (uint32_t)(std::upper_bound(a + 1, a + n, u, [](double x, float y) { return x < (double)y; }) - a) - 1u;
+}
+static inline double cdf_step(const float* a, uint32_t n, uint32_t k) { return (k + 1u < n ? (double)a[k + 1u] : 1.) - (double)a[k]; }
+
+static inline double env_cell_pdf(const EnvTable& e, uint32_t i, uint32_t j) {
+    const double pm = cdf_step(e.marg.data(), e.ch, i), pc = cdf_step(e.cond.data() + (size_t)i * e.cw, e.cw, j);
+    return pm * pc * (double)e.inv_dphi / (double)e.dcos[i];
+}
+
+// the cell Scene::background reads direction dir from
+static inline void env_cell_of(const Scene& s, const EnvTable& e, V3 dir, uint32_t& i, uint32_t& j) {
+    dir = unit(dir);
+    const double x = (std::atan2(dir.z, dir.x) + PI) / (2. * PI) * (double)(s.hdri_w - 1);
+    const double y = std::acos(std::fmin(1., std::fmax(-1., dir.y))) / PI * (double)(s.hdri_h - 1);
+    j = std::min((uint32_t)std::floor(x), e.cw - 1u);
+    i = std::min((uint32_t)std::floor(y), e.ch - 1u);
+}
+
+static inline double env_pdf(const Scene& s, const EnvTable& e, V3 dir) {
+    if (e.marg.empty()) return 0.;
+    uint32_t i, j;
+    env_cell_of(s, e, dir, i, j);
+    return env_cell_pdf(e, i, j);
+}
+
+// (hi0, hi1): multiples of 2^-24 that pick the row and the cell; hi + 2^-24 lo places the direction inside it.
+// Returns the density of the drawn cell.
+static inline double env_sample(const EnvTable& e, double hi0, double hi1, double lo0, double lo1, V3& dir, uint32_t& i,
+                                uint32_t& j) {
+    i = cdf_find(e.marg.data(), e.ch, hi0);
+    const double pm = cdf_step(e.marg.data(), e.ch, i);
+    const float* cond = e.cond.data() + (size_t)i * e.cw;
+    j = cdf_find(cond, e.cw, hi1);
+    const double pc = cdf_step(cond, e.cw, j);
+    const double t0 = std::fmin(((hi0 - (double)e.marg[i]) + lo0 / 16777216.0) / pm, 1.);
+    const double t1 = std::fmin(((hi1 - (double)cond[j]) + lo1 / 16777216.0) / pc, 1.);
+    const double cy = (double)e.cos0[i] - t0 * (double)e.dcos[i];
+    const double sy = std::sqrt(std::fmax(0., (1. - cy) * (1. + cy)));
+    const double phi = 2. * PI * ((double)j + t1) / (double)e.cw;
+    dir = v3(-sy * std::cos(phi), cy, -sy * std::sin(phi));
+    return env_cell_pdf(e, i, j);
+}
+
+// a uniform in [0, 1) split as the device draws it: the 24-bit part that picks the cell and the rest (in [0, 1))
+static inline void env_split(double u, double& hi, double& lo) {
+    const double x = std::ldexp(std::fmin(std::fmax(u, 0.), 1.), 24);
+    const double f = std::fmin(std::floor(x), 16777215.);
+    hi = std::ldexp(f, -24);
+    lo = std::fmin(x - f, 1.);
+}
+
+// env.cuh nee_bsdf: W = the plain estimator's weight for direction l, return = the density with which the plain
+// render produces l (0: never).  Cook-Torrance: Beckmann D from tan^2 = |n x h|^2 / nh^2, 0 from tan^2 / alpha^2 >= 80
+// on (the device's cut-off), half-vector density D cos theta_h mirrored (1 / (4 h.v)).
+static inline double nee_bsdf(const Material& m, V3 n, V3 v, V3 l, V3& W) {
+    W = v3(0., 0., 0.);
+    if (m.tag == MAT_LAMBERTIAN) {
+        const double nl = dot(n, l);
+        if (!(nl > 0.)) return 0.;
+        W = m.color;
+        return nl * FRAC_1_PI;
+    }
+    const V3 hh = v + l;
+    if (is_zeros(hh)) return 0.;
+    const V3 h = unit(hh);
+    const double nh = dot(n, h), hv = dot(h, v), nl = dot(n, l), nv = std::fabs(dot(n, v));
+    if (!(nh > 0.) || !(hv > 0.) || nl <= 0. || nv == 0.) return 0.;
+    const double g = rmin(2. * nh * nv / hv, rmin(2. * nh * nl / hv, 1.));
+    const V3 F = fresnel_value(m, m.fresnel_kind, h, v, ENTERING);
+    W = m.color * F * (g * dot(h, l) / nv);
+    const V3 c = cross(n, h);
+    const double t = dot(c, c) / (nh * nh * m.alpha2);
+    if (!(t < 80.)) return 0.;
+    const double nh2 = nh * nh;
+    return std::exp(-t) / (PI * m.alpha2 * nh2 * nh2) * nh / (4. * hv);
+}
+
+// power heuristic a^2 / (a^2 + b^2) and the cross term a b / (a^2 + b^2), at least one of a, b positive
+static inline double mis_power(double a, double b) {
+    const double s = rmin(a, b) / rmax(a, b), s2 = s * s;
+    return (a >= b ? 1. : s2) / (1. + s2);
+}
+static inline double mis_cross(double a, double b) {
+    const double s = rmin(a, b) / rmax(a, b);
+    return s / (1. + s * s);
+}
+
 struct PathStats {
-    uint64_t rays = 0;        // Bvh::intersect calls
+    uint64_t rays = 0;        // Bvh::intersect calls (shadow rays included)
+    uint64_t shadow_rays = 0; // of which environment shadow rays
     uint64_t scatters = 0;
     uint64_t nan_pixels = 0;
     uint64_t neg_pixels = 0;
@@ -978,11 +1155,16 @@ struct PathStats {
     uint64_t reentry_lost = 0;
 };
 
-// radiance lib.rs:521-560
-static V3 radiance(const Scene& s, Ray r, uint32_t max_bounces, Rng& rng, PathStats& st) {
+// radiance lib.rs:521-560.  env != nullptr: with next-event estimation of the environment as the GPU backend's
+// RRS_FLAG_ENV_SAMPLING does it (wavefront.cu shade_hit / env_miss): at a Lambertian vertex or a Cook-Torrance vertex
+// with alpha^2 > 0 in fp32, below the last bounce, one direction from the table (RNG slot 0x100 + b) is traced as a
+// shadow ray and adds throughput * W * background * min(p, 1) / p * mis_cross(p_e, p_b) if it escapes; the
+// continuation's escape is weighted by mis_power(p_b, p_e) (1 where the shadow strategy cannot produce its direction).
+static V3 radiance(const Scene& s, Ray r, uint32_t max_bounces, Rng& rng, PathStats& st, const EnvTable* env = nullptr) {
     V3 throughput = v3(1., 1., 1.);
     V3 light = v3(0., 0., 0.);
     const Object* origin_obj = nullptr;
+    double wcont = 1.;  // MIS weight of the current ray's escape
     for (uint32_t b = 0; b < max_bounces; ++b) {
         st.rays++;
         Hit h = tree_intersect(s.bvh.get(), r, s.tmin, s.tmax);
@@ -1001,7 +1183,29 @@ static V3 radiance(const Scene& s, Ray r, uint32_t max_bounces, Rng& rng, PathSt
             V3 view = unit(-1. * r.d);
             rng.load(b + 1);
             DrawSrc rs{rng.u, 0};
-            ScatterEvent e = material_evaluate(s.materials[h.obj->mat], position, normal, view, rs);
+            const Material& mat = s.materials[h.obj->mat];
+            ScatterEvent e = material_evaluate(mat, position, normal, view, rs);
+            const bool nee = env && !env->marg.empty() && b + 1 < max_bounces &&
+                             (mat.tag == MAT_LAMBERTIAN || (mat.tag == MAT_COOK_TORRANCE && (float)mat.alpha2 > 0.f));
+            if (nee) {
+                Rng re = rng;
+                re.load(0x100u + b);
+                double hi0 = re.u[0], hi1 = re.u[1], lo0 = re.u[2], lo1 = re.u[3];
+                if (rng.mode != 1) { env_split(re.u[0], hi0, lo0); env_split(re.u[1], hi1, lo1); }
+                V3 l, W;
+                uint32_t ci, cj;
+                const double pe = env_sample(*env, hi0, hi1, lo0, lo1, l, ci, cj);
+                const double pb = pe > 0. ? nee_bsdf(mat, normal, view, l, W) : 0.;
+                const V3 tw = throughput * W;
+                const double p = rmax(rmax(tw.x, tw.y), tw.z);
+                if (pb > 0. && p > 0.) {
+                    const double k = rmin(p, 1.) / p * mis_cross(pe, pb);
+                    st.rays++;
+                    st.shadow_rays++;
+                    if (!tree_intersect(s.bvh.get(), Ray{position, l}, s.tmin, s.tmax).hit)
+                        light = light + tw * s.background(l) * k;
+                }
+            }
             if (e.scatter) {
                 st.scatters++;
                 V3 emit = h.obj->emission < 0 ? v3(0, 0, 0) : s.emissions[h.obj->emission].emit();
@@ -1012,10 +1216,19 @@ static V3 radiance(const Scene& s, Ray r, uint32_t max_bounces, Rng& rng, PathSt
                 // DivAssign<f64> is a true per-component division vecmath.rs:708-714
                 throughput.x /= p; throughput.y /= p; throughput.z /= p;
                 r = e.ray;
+                if (nee) {
+                    V3 W;
+                    const double pb = nee_bsdf(mat, normal, view, r.d, W);
+                    const double pe = env_pdf(s, *env, r.d);
+                    wcont = pe > 0. && pb > 0. ? mis_power(pb, pe) : 1.;
+                } else {
+                    wcont = 1.;
+                }
             } else {
                 return light;
             }
         } else {
+            if (env) return light + throughput * wcont * s.background(r.d);
             return light + throughput * s.background(r.d);
         }
     }
@@ -1031,6 +1244,7 @@ using namespace orc;
 
 struct OrcScene {
     Scene s;
+    EnvTable env;  // the environment-sampling table of s's HDRI
     std::string err;
 };
 
@@ -1082,6 +1296,7 @@ OrcScene* orc_scene_create(const double* objs, uint64_t n_obj, const double* mat
     s.hdri_h = hh;
     s.hdri.resize(hw * hh);
     for (uint64_t i = 0; i < hw * hh; ++i) s.hdri[i] = v3(hdri[i * 3], hdri[i * 3 + 1], hdri[i * 3 + 2]);
+    build_env_table(s.hdri, hw, hh, h->env);
     // Bvh::build bvh.rs:199-210 -> BvhData::new :87-98
     std::vector<const Object*> ptrs(n_obj);
     std::vector<V3> centers(n_obj);
@@ -1238,9 +1453,10 @@ void orc_primary_rays(const double* cam17, uint32_t W, uint32_t H, const uint32_
 
 // The render call being replaced: rayrs/src/main.rs:52-94.  out: H x W x 3 mean radiance.
 // stats_out: [rays, scatters, nan_pixels, negative_pixels, seconds*1e6, reentry_total, reentry_lost]
-void orc_render(const OrcScene* h, const double* cam17, uint32_t W, uint32_t H, uint32_t spp,
-                uint32_t sample_offset, uint32_t max_bounces, uint64_t seed, int rng_mode, int nthreads,
-                double* out, uint64_t* stats_out) {
+// env: with environment sampling (radiance); stats_out then has an 8th entry, the shadow rays (counted in rays too).
+static void render(const OrcScene* h, const double* cam17, uint32_t W, uint32_t H, uint32_t spp, uint32_t sample_offset,
+                   uint32_t max_bounces, uint64_t seed, int rng_mode, int nthreads, double* out, uint64_t* stats_out,
+                   const EnvTable* env) {
     const Scene& s = h->s;
     Camera c = camera_from_derived(cam17);
     const uint32_t B = 16;  // main.rs:57
@@ -1264,7 +1480,7 @@ void orc_render(const OrcScene* h, const double* cam17, uint32_t W, uint32_t H, 
                         Rng rng{seed, row * W + col, sample_offset + k, rng_mode, {0, 0, 0, 0}};
                         rng.load(0);
                         Ray r = camera_primary_ray(c, (size_t)H - i - off_y, (size_t)W - j - off_x, rng.u[0], rng.u[1]);
-                        pixel = pixel + radiance(s, r, max_bounces, rng, st);
+                        pixel = pixel + radiance(s, r, max_bounces, rng, st, env);
                     }
                     if (std::isnan(pixel.x) || std::isnan(pixel.y) || std::isnan(pixel.z)) st.nan_pixels++;
                     if (pixel.x < 0. || pixel.y < 0. || pixel.z < 0.) st.neg_pixels++;
@@ -1285,6 +1501,7 @@ void orc_render(const OrcScene* h, const double* cam17, uint32_t W, uint32_t H, 
             tot.rays += st.rays; tot.scatters += st.scatters;
             tot.nan_pixels += st.nan_pixels; tot.neg_pixels += st.neg_pixels;
             tot.reentry_total += st.reentry_total; tot.reentry_lost += st.reentry_lost;
+            tot.shadow_rays += st.shadow_rays;
         }
         stats_out[0] = tot.rays;
         stats_out[1] = tot.scatters;
@@ -1293,7 +1510,62 @@ void orc_render(const OrcScene* h, const double* cam17, uint32_t W, uint32_t H, 
         stats_out[4] = (uint64_t)std::chrono::duration_cast<std::chrono::microseconds>(t1 - t0).count();
         stats_out[5] = tot.reentry_total;
         stats_out[6] = tot.reentry_lost;
+        if (env) stats_out[7] = tot.shadow_rays;
     }
+}
+
+void orc_render(const OrcScene* h, const double* cam17, uint32_t W, uint32_t H, uint32_t spp,
+                uint32_t sample_offset, uint32_t max_bounces, uint64_t seed, int rng_mode, int nthreads,
+                double* out, uint64_t* stats_out) {
+    render(h, cam17, W, H, spp, sample_offset, max_bounces, seed, rng_mode, nthreads, out, stats_out, nullptr);
+}
+
+// orc_render with environment sampling (RRS_FLAG_ENV_SAMPLING).  stats_out: 8 entries, the last the shadow rays.
+// Returns -1 (and renders nothing) if the map has a non-finite texel, as the GPU backend refuses the flag.
+int orc_render_env(const OrcScene* h, const double* cam17, uint32_t W, uint32_t H, uint32_t spp, uint32_t sample_offset,
+                   uint32_t max_bounces, uint64_t seed, int rng_mode, int nthreads, double* out, uint64_t* stats_out) {
+    if (!h->env.ok) return -1;
+    render(h, cam17, W, H, spp, sample_offset, max_bounces, seed, rng_mode, nthreads, out, stats_out, &h->env);
+    return 0;
+}
+
+// The sampling table: returns 1 (tabulated), 0 (black map: empty table) or -1 (non-finite texels).  Each of marg
+// (ch floats), cond (ch x cw floats) and row (ch x 2 floats: cos theta at the top edge, cos top - cos bottom) may be
+// null; they are written only for a tabulated map.
+int orc_env_table(const OrcScene* h, float* marg, float* cond, float* row) {
+    const EnvTable& e = h->env;
+    if (!e.ok) return -1;
+    if (e.marg.empty()) return 0;
+    if (marg) std::memcpy(marg, e.marg.data(), sizeof(float) * e.marg.size());
+    if (cond) std::memcpy(cond, e.cond.data(), sizeof(float) * e.cond.size());
+    if (row)
+        for (uint32_t i = 0; i < e.ch; ++i) { row[2 * i] = e.cos0[i]; row[2 * i + 1] = e.dcos[i]; }
+    return 1;
+}
+
+// rrs_env_sample's inputs: u n x 2 uniforms in [0, 1), each split into the 24 bits that pick the cell and the rest.
+// out: n x 6 = direction xyz, density of the drawn cell, cell row, cell column.  -1 if the table is empty or refused.
+int orc_env_sample(const OrcScene* h, const double* u, uint64_t n, double* out) {
+    const EnvTable& e = h->env;
+    if (!e.ok || e.marg.empty()) return -1;
+    for (uint64_t k = 0; k < n; ++k) {
+        double hi0, lo0, hi1, lo1;
+        env_split(u[2 * k], hi0, lo0);
+        env_split(u[2 * k + 1], hi1, lo1);
+        V3 d;
+        uint32_t i, j;
+        const double pdf = env_sample(e, hi0, hi1, lo0, lo1, d, i, j);
+        double v[6] = {d.x, d.y, d.z, pdf, (double)i, (double)j};
+        std::memcpy(out + 6 * k, v, sizeof(v));
+    }
+    return 0;
+}
+
+// rrs_env_pdf: the density of n directions (n x 3) in the cell background() reads them from.  -1 if refused.
+int orc_env_pdf(const OrcScene* h, const double* dirs, uint64_t n, double* pdf) {
+    if (!h->env.ok) return -1;
+    for (uint64_t k = 0; k < n; ++k) pdf[k] = env_pdf(h->s, h->env, v3(dirs[3 * k], dirs[3 * k + 1], dirs[3 * k + 2]));
+    return 0;
 }
 
 // Material::evaluate for a batch.  mat_row: 12 doubles.  nv: n x 6 (normal, view — both unit).

@@ -131,6 +131,12 @@ static void build_env_table(const std::vector<float4>& hdri, uint32_t w, uint32_
         const float4 t = hdri[(size_t)i * w + j];
         return std::max(std::fabs(t.x), std::max(std::fabs(t.y), std::fabs(t.z)));
     };
+    // a NaN in a texel's second or third channel would vanish in std::max below: check every channel first
+    for (const float4& t : hdri)
+        if (!std::isfinite(t.x) || !std::isfinite(t.y) || !std::isfinite(t.z)) {
+            out.env_ok = false;
+            return;
+        }
     std::vector<double> cell((size_t)cw * ch), rows(ch);
     out.env_row.resize(ch);
     const double dphi = 2. * M_PI / cw;

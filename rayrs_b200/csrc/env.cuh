@@ -62,7 +62,9 @@ __device__ __forceinline__ float env_pdf(const DScene& sc, const DEnv& e, float3
 
 // Draw a direction.  (u0, u1) pick the row and the cell (24-bit uniforms, as the device RNG hands them out);
 // (u0 + 2^-24 * lo0, u1 + 2^-24 * lo1) as 48-bit uniforms place the direction inside the cell, so that the position
-// stays continuous even in a cell one CDF step wide.  Returns env_pdf of the direction.
+// stays continuous even in a cell one CDF step wide.  Returns the density of the drawn cell: the density the sampler
+// realises.  (env_pdf of the fp32 direction can read a neighbouring cell when the direction lies within rounding of
+// the cell's edge, and a neighbour 10^6 times dimmer, or black, would turn the shadow ray's weight into a spike.)
 __device__ __forceinline__ float env_sample(const DScene& sc, const DEnv& e, float u0, float u1, float lo0, float lo1,
                                             float3& dir) {
     const uint32_t i = cdf_find(e.marg, e.ch, u0);
@@ -78,7 +80,7 @@ __device__ __forceinline__ float env_sample(const DScene& sc, const DEnv& e, flo
     float sp, cp;
     sincospif(2.f * ((float)j + t1) / (float)e.cw, &sp, &cp);
     dir = f3(-sy * cp, cy, -sy * sp);  // phi = atan2(z, x) + pi, theta = acos(y)
-    return env_pdf(sc, e, dir);
+    return pm * pc * e.inv_dphi / r.y;  // env_cell_pdf(e, i, j)
 }
 
 // Beckmann D(h) for cos theta_h = nh, with tan^2 from |n x h|^2 (no cancellation at alpha = 0.01)

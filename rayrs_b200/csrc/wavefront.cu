@@ -526,7 +526,9 @@ __device__ __forceinline__ NextRay shade_hit(const DScene& sc, const RenderConst
                 float3 W;
                 const float pb = nee_bsdf(m, mtag, nrm, view, so.dir, W);
                 const float pe = env_pdf(sc, *env, so.dir);
-                *wcont = pe > 0.f ? mis_power(pb, pe) : 1.f;
+                // pb == 0 in fp32 (a direction at grazing incidence, or beyond beckmann_d's cut-off): the shadow ray
+                // never contributes in this direction, so the continuation carries all of it
+                *wcont = pe > 0.f && pb > 0.f ? mis_power(pb, pe) : 1.f;
             }
         }
     }

@@ -264,7 +264,10 @@ def test_probes_match_the_restatement(which, native_built):
     near_edge = np.any((tt < 1e-4) | (tt > 1 - 1e-4), axis=1)  # the fp32 lookup may read the neighbour cell
     rel = np.abs(got[:, 3] - ref) / ref
     assert np.all(rel[~near_edge] < 1e-4) and near_edge.mean() < 1e-2
-    assert np.array_equal(sc.env_pdf(got[:, :3]), got[:, 3])            # round trip, bit for bit
+    assert np.all(rel < 1e-6)       # the sampler returns the density of the cell it drew, at a cell edge too
+    # round trip, bit for bit, wherever the fp32 direction reads back the cell it was drawn in
+    back = sc.env_pdf(got[:, :3])
+    assert np.array_equal(back[~near_edge], got[~near_edge, 3]) and (back != got[:, 3]).mean() < 1e-3
     d = rng.normal(size=(20000, 3))
     p = sc.env_pdf(d)
     x, y = t.coords(d)
